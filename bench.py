@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — node expansions/s of the batched PA-Star search on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[3], synthetic N=7 x length 500 random protein (seed 12345),
@@ -16,6 +16,8 @@ roofline = the round's dominant kernel (expand + probe) against the measured HBM
          roofline.kernels lists select / claim / expand+probe / insert with their CUDA-event times and algorithmic bytes.
 cpu_baseline / --impl reference = the reference's own getNeigh / PairAlign / weights (oracle/_ref, compiled from
          the unmodified sources) under the restated T-thread hash-partitioned driver, on this box's host cores.
+--dump-outputs DIR (N = 1) = after the K timed rounds, what they leave a caller of the search (see search_outputs) as
+         DIR/<name>.npy in float64, so that two builds can be compared output for output on identical inputs.
 """
 import argparse
 import json
@@ -45,6 +47,27 @@ def s7_seqs():
     import random
     r = random.Random(SEED)
     return ["".join(r.choice(AA) for _ in range(LENGTH)) for _ in range(N_SEQ)]
+
+
+STATUS_FIELDS = ("finished", "g", "f", "pops", "expansions", "generated", "reopen", "open_size", "closed_size", "rounds",
+                 "probed", "pushed", "inserted", "survivors")  # pg_result counters; the timing fields are left out
+DUMP_NODES, DUMP_DEPTH = 4096, 4
+
+
+def search_outputs(G):
+    """What the search rounds so far give their caller: pg_search_status (min open f, best goal g, counters) and, through
+    pg_search_lookup, the g and parenti (-1 when absent) of DUMP_NODES lattice nodes within DUMP_DEPTH moves of the
+    start, drawn with a fixed seed.  The min open f and the values of settled nodes (g + h below the min open f: closed
+    with their final g; all of the sample in the default configuration) repeat exactly from run to run; pops, expansions
+    and the other counters vary in about the fifth digit, because concurrent inserts of one node race to the table."""
+    min_f, goal, c = G.search_status()
+    rng = np.random.default_rng(SEED)
+    moves = rng.integers(1, 1 << G.n, (DUMP_NODES, DUMP_DEPTH))
+    moves[np.arange(DUMP_DEPTH) >= rng.integers(1, DUMP_DEPTH + 1, (DUMP_NODES, 1))] = 0
+    pos = ((moves[:, :, None] >> np.arange(G.n)) & 1).sum(axis=1).astype(np.uint16)
+    vals = np.array([G.search_lookup(p) or (-1, -1) for p in pos], dtype=np.float64).reshape(DUMP_NODES, 2)
+    return {"search_status": np.array([min_f, goal] + [c[k] for k in STATUS_FIELDS], dtype=np.float64),
+            "node_pos": pos.astype(np.float64), "node_g": vals[:, 0], "node_parenti": vals[:, 1]}
 
 
 def measured_peaks():
@@ -154,7 +177,7 @@ def run_reference(args, rank, world):
     if rank != 0:
         return
     threads = os.cpu_count() or 1
-    steps = max(1, args.steps)
+    steps = args.steps
     t0 = time.time()
     b = cpu_reference_run(threads, steps, args.warmup)
     line = {"impl": "reference", "metric": METRIC, "value": b["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
@@ -249,7 +272,7 @@ def run_ours(args, rank, world):
 
     seqs = s7_seqs()
     batch, cap = args.batch, args.table_capacity
-    K, W = max(1, args.steps), max(3, args.warmup)
+    K, W = args.steps, max(3, args.warmup)
     stream = torch.cuda.current_stream()
 
     G = m.PastarGPU(seqs, device=local)
@@ -291,6 +314,10 @@ def run_ours(args, rank, world):
         v1 = G.search_status()[2]
         total_exp = v1["expansions"] - v0["expansions"]
         dv = {k: v1[k] - v0[k] for k in ("expansions", "generated", "probed", "pushed", "pops")}
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in search_outputs(G).items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         # ---- pass 2, the per-kernel times behind `roofline`: the next K rounds with an event pair around every launch
         # (plain launches: the extra events would sit between graph nodes)
         c0 = G.search_status()[2]
@@ -712,9 +739,14 @@ def main():
                          "coordinates: an eighth of the parents straddle a partition boundary per owner coordinate; FZORDER shift 12 "
                          "(bit 1 of five coordinates) makes most parents straddle several")
     ap.add_argument("--no-hash-sweep", action="store_true", help="N > 1: skip the FZORDER shift 12 / 17 comparison runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="N = 1: write what the timed rounds computed as DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     if args.impl == "reference":
         run_reference(args, rank, world)
     else:

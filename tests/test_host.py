@@ -61,10 +61,11 @@ def test_read_fasta_rules(tmp_path):
     p = tmp_path / "x.fasta"
     p.write_text(">a\nAC\nGT\n\n>b\nTT\n>c\n>d\nGG")  # '>' and empty lines end a record; empty records are dropped
     assert m.read_fasta(str(p)) == ["ACGT", "TT", "GG"]
-    for name in ("test", "test2", "PF08184", "kinase"):
-        src = os.path.join("/root/reference", name + ".fasta")
-        if os.path.exists(src):
-            assert m.read_fasta(src) == CASES[name]
+    for name in ("test", "test2", "PF08184", "kinase"):  # the reference fixtures, written as multi-line records
+        src = tmp_path / (name + ".fasta")
+        src.write_text("".join(">%s_%d\n%s\n" % (name, i, "\n".join(q[k:k + 60] for k in range(0, len(q), 60)))
+                               for i, q in enumerate(CASES[name])))
+        assert m.read_fasta(str(src)) == CASES[name]
 
 
 @pytest.mark.skipif(has_gpu(), reason="checks the no-GPU failure mode")
@@ -104,14 +105,12 @@ def _weight_edge_cases():
 def test_host_weights_edge_cases_vs_reference_build(name):
     """pg_host_weights against the reference compiled in place (oracle/_ref), float bit patterns, on inputs the golden
     file does not hold: ragged lengths down to 1, every supported N, identical sequences (zero distances), two distant
-    groups (the reference's weights overflow to inf there, and so must ours), letters with unset PAM rows."""
-    from oracle import refio
-    if not refio.available():
-        pytest.skip("oracle/_ref is built by __graft_entry__.build() where /root/reference exists")
+    groups (the reference's weights overflow to inf there, and so must ours), letters with unset PAM rows.  Without the
+    build the reference's bit patterns come from tests/golden/ref_comparisons.json.gz (tests/refdata.py)."""
+    import refdata
     seqs = _weight_edge_cases()[name]
-    ref = refio.dump(seqs)["weights"]
     w = m.host_weights(seqs)
-    assert np.array_equal(w.view(np.uint32), ref.view(np.uint32))
+    assert w.view(np.uint32).ravel().tolist() == refdata.dump(seqs)["weights"]
 
 
 def test_host_weights_refuses_residues_outside_the_cost_table():
