@@ -252,6 +252,23 @@ int pg_search_status(pg_ctx *ctx, int32_t *min_open_f, int32_t *best_goal_g, pg_
  * (pastar_functions/PAStarDistributedBacktrace.cpp:18-214): found=0 if absent. */
 int pg_search_lookup(pg_ctx *ctx, const uint16_t *pos, int32_t *found, int32_t *g, int32_t *parenti);
 int pg_search_end(pg_ctx *ctx);
+/* Bounded-suboptimal (weighted) search - an opt-in extension of pg_search / pg_multi_search / pg_search_begin (the
+ * reference, PAStar.cpp:626-673, only searches for the optimum).  Every later search on the context orders, prunes and
+ * stops on f_w = g + h_w, h_w = sum over pairs of floor(num * w_ij * T_ij / den), h <= h_w <= (num/den) h, and returns an
+ * alignment that costs at most num/den times the optimum.  den is a power of two in 1..1024, den <= num <= 16 den;
+ * (1, 1), the default, is the exact search and leaves every result unchanged.  pg_expand_batch and pg_calculate_h stay
+ * unweighted.  With num > den the reported g = f is the re-scored cost of the alignment returned (its parent chain may be
+ * cheaper than the best goal found).  PG_ERR_ARG for a bad weight, PG_ERR_STATE while a step-wise search is active;
+ * pg_multi_search refuses contexts whose weights differ (PG_ERR_ARG), and pg_search_begin refuses, with
+ * PG_ERR_UNSUPPORTED, a weighted f range beyond 2^27 buckets. */
+int pg_search_set_weight(pg_ctx *ctx, int32_t num, int32_t den);
+/* Certified lower bound on the optimal cost: the minimum of g + h over the open entries, of g + h over the successors a
+ * weighted search dropped, of the best goal and of the all-advance cost.  After pg_search / pg_multi_search: the bound of
+ * that search (every context of a pg_multi_search reports the global one); a finished search has g * den <= num * bound
+ * (an exact search: bound == g), a budgeted one bound <= optimum.  While a step-wise search is active: this partition's
+ * bound, computed now (the driver takes the minimum over the partitions between rounds).  PG_ERR_STATE before any
+ * search. */
+int pg_search_lower_bound(pg_ctx *ctx, int32_t *lower_bound);
 /* bytes per exchanged successor record for this context */
 int pg_xrec_stride(const pg_ctx *ctx);
 

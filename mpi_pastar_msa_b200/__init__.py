@@ -9,4 +9,4 @@ but every compute call needs the built library and a CUDA device and fails loudl
 otherwise.
 """
 from .api import (HASH_TYPES, allow_extended_n, release_cached_memory, bench_random_gather, bench_int_peak, PastarError, PastarGPU, default_cost_table, gpu_weights, host_weights, lib_path, load_library, multi_search,  # noqa: F401
-                  node_dtype, read_fasta, rescore_alignment, succ_dtype)
+                  node_dtype, read_fasta, rescore_alignment, succ_dtype, WEIGHT_DEN, weight_fraction)

@@ -9,8 +9,10 @@ Reference interface                                   -> here
   Coord::configure_hash / get_id (CoordHash.cpp)       -> .configure_hash / .owner
   Node::getNeigh (Node.cpp:205-248)                    -> .expand_batch / .get_neigh
   PAStar::pa_star (PAStar.cpp:626-673)                 -> .search
+  (no reference counterpart: bounded-suboptimal search) -> .search(weight=W) / .search_set_weight / .search_lower_bound
 """
 import ctypes as C
+import math
 import os
 
 import numpy as np
@@ -107,6 +109,8 @@ def load_library():
         "pg_search_lookup": ([vp, vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)], i32),
         "pg_search_end": ([vp], i32),
         "pg_xrec_stride": ([vp], i32),
+        "pg_search_set_weight": ([vp, C.c_int32, C.c_int32], i32),
+        "pg_search_lower_bound": ([vp, C.POINTER(C.c_int32)], i32),
     }
     for name, (args, res) in sig.items():
         f = getattr(L, name)
@@ -121,7 +125,14 @@ EXPORTS = ["pg_release_cached_memory", "pg_search_note_rounds", "pg_search_set_d
            "pg_build_pair_tables", "pg_pair_table_shape", "pg_copy_pair_table", "pg_calculate_h", "pg_configure_hash",
            "pg_owner", "pg_expand_batch", "pg_expand_batch_dev", "pg_search", "pg_search_begin", "pg_search_round",
            "pg_search_outbox", "pg_search_insert_dev", "pg_search_status", "pg_search_lookup", "pg_search_end",
-           "pg_xrec_stride"]
+           "pg_xrec_stride", "pg_search_set_weight", "pg_search_lower_bound"]
+
+WEIGHT_DEN = 1024
+
+
+def weight_fraction(weight):
+    """Search weight W (1 <= W <= 16) as (num, den): num / 1024 rounded up, as the pastar CLI's --weight."""
+    return int(math.ceil(float(weight) * WEIGHT_DEN)), WEIGHT_DEN
 
 
 def node_dtype(n):
@@ -174,12 +185,16 @@ def bench_random_gather(nbytes, device=-1):
     return out.value
 
 
-def multi_search(gpus, table_capacity=0, batch_target=0, max_expansions=0, rounds_per_sync=0, want_rows=True):
+def multi_search(gpus, table_capacity=0, batch_target=0, max_expansions=0, rounds_per_sync=0, want_rows=True, weight=1.0):
     """pg_multi_search: one hash-owned partition per context in `gpus` (PastarGPU objects with their pair tables built and
     the same hash configuration; normally one per device, but contexts on one device work too), driven by this process.
-    Returns (total dict, list of per-partition dicts)."""
+    weight != 1: bounded-suboptimal search (see PastarGPU.search), set on every context.
+    Returns (total dict with lower_bound / weight_num / weight_den, list of per-partition dicts)."""
     L = load_library()
     g0 = gpus[0]
+    if weight != 1.0:
+        for g in gpus:
+            g.search_set_weight(*weight_fraction(weight))
     cfg = SearchConfig(len(gpus), 0, table_capacity, batch_target, max_expansions, rounds_per_sync, 0)
     res, parts = Result(), (Result * len(gpus))()
     handles = (C.c_void_p * len(gpus))(*[g.h for g in gpus])
@@ -192,6 +207,8 @@ def multi_search(gpus, table_capacity=0, batch_target=0, max_expansions=0, round
     d = res.as_dict()
     if want_rows and res.finished:
         d["rows"] = [b.value.decode() for b in bufs]
+    d["lower_bound"] = g0.search_lower_bound()
+    d["weight_num"], d["weight_den"] = g0.weight
     return d, [p.as_dict() for p in parts]
 
 
@@ -308,6 +325,7 @@ class PastarGPU:
                 self.h = None
             raise PastarError(rc, msg)
         self.tables_ms = None
+        self.weight = (1, 1)  # (num, den) of the search weight last set on the context
 
     def close(self):
         if getattr(self, "h", None):
@@ -388,7 +406,11 @@ class PastarGPU:
         return s[np.argsort(s["owner"], kind="stable")]
 
     # ---- (3)+(4) search
-    def search(self, table_capacity=0, batch_target=0, max_expansions=0, rounds_per_sync=0, want_rows=True):
+    def search(self, table_capacity=0, batch_target=0, max_expansions=0, rounds_per_sync=0, want_rows=True, weight=1.0):
+        """weight W > 1: bounded-suboptimal search (num / 1024 rounded up, as the CLI's --weight): g <= W x the optimum,
+        certified by the returned lower_bound (g * weight_den <= weight_num * lower_bound when finished)."""
+        if weight != 1.0:
+            self.search_set_weight(*weight_fraction(weight))
         cfg = SearchConfig(1, 0, table_capacity, batch_target, max_expansions, rounds_per_sync, 0)
         res = Result()
         rows, bufs = None, None
@@ -400,7 +422,22 @@ class PastarGPU:
         d = res.as_dict()
         if want_rows and res.finished:
             d["rows"] = [b.value.decode() for b in bufs]
+        d["lower_bound"] = self.search_lower_bound()
+        d["weight_num"], d["weight_den"] = self.weight
         return d
+
+    def search_set_weight(self, num, den):
+        """pg_search_set_weight: every later search on this context is weighted by num / den (den a power of two <= 1024,
+        den <= num <= 16 den); (1, 1) is the exact search."""
+        self._ck(self.L.pg_search_set_weight(self.h, int(num), int(den)))
+        self.weight = (int(num), int(den))
+
+    def search_lower_bound(self):
+        """pg_search_lower_bound: certified lower bound on the optimal cost (of the last search, or of this partition of
+        the active step-wise search)."""
+        v = C.c_int32()
+        self._ck(self.L.pg_search_lower_bound(self.h, C.byref(v)))
+        return v.value
 
     # step-wise (multi-GPU drivers)
     def search_begin(self, n_parts=1, part=0, table_capacity=0, batch_target=0, p2p=False):

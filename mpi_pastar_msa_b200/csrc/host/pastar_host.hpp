@@ -19,6 +19,7 @@
 #include <unistd.h>
 
 #include <chrono>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -406,6 +407,7 @@ struct PAStarOpt { // PAStar.h:87-112, plus the GPU-side knobs (new, do not chan
     int gpus = 1;
     long long batch = 0, table_capacity = 0, max_expansions = 0;
     std::string metrics_json; // --metrics_json FILE: counters of the run as one JSON object (PAStarSyncData.cpp's gather, machine-readable)
+    int weight_num = 0;       // --weight W: bounded-suboptimal search with weight weight_num / 1024 (0 = not given: exact search)
 };
 
 int read_fasta_file(const std::string &name);
@@ -442,25 +444,41 @@ class PAStar {
         std::vector<std::vector<char>> bufs(N, std::vector<char>(total));
         std::vector<char *> rowp(N);
         for (int i = 0; i < N; i++) rowp[i] = bufs[i].data();
+        const int wden = 1024;
+        int32_t lower_bound = 0;
         if (gpus == 1) {
+            if (options.weight_num) h->check(pg_search_set_weight(h->ctx, options.weight_num, wden), "pg_search_set_weight");
             TimeCounter t("Phase 2: PA-Star running time: ");
             h->check(pg_search(h->ctx, &cfg, &res, rowp.data()), "pg_search");
             parts[0] = res;
+            if (options.weight_num) h->check(pg_search_lower_bound(h->ctx, &lower_bound), "pg_search_lower_bound");
         } else {
             // one hash-owned partition per GPU (the reference: one per thread x MPI rank, PAStar.cpp:107-117)
             std::vector<pg_ctx *> ctxs = h->contexts(gpus);
             for (pg_ctx *c : ctxs) h->check(pg_configure_hash(c, (int)options.hash_type, options.hash_shift), "pg_configure_hash");
+            if (options.weight_num)
+                for (pg_ctx *c : ctxs) h->check(pg_search_set_weight(c, options.weight_num, wden), "pg_search_set_weight");
             TimeCounter t("Phase 2: PA-Star running time: ");
             h->check(pg_multi_search(ctxs.data(), gpus, &cfg, &res, parts.data(), rowp.data()), "pg_multi_search");
+            if (options.weight_num) h->check(pg_search_lower_bound(ctxs[0], &lower_bound), "pg_search_lower_bound");
         }
+        // weighted search: the optimum is at least the lower bound, so g / bound is the certified ratio to it
+        auto print_bound = [&]() {
+            if (options.weight_num <= wden) return;
+            std::cout << "Lower bound: " << lower_bound;
+            if (res.finished) std::cout << "\tg / lower bound: " << std::fixed << std::setprecision(4) << (double)res.g / lower_bound;
+            std::cout << std::endl;
+        };
         if (!res.finished) {
             std::cout << "Search stopped at the expansion budget: " << res.expansions << " expansions, no alignment.\n";
+            print_bound();
         } else {
             TimeCounter *t = new TimeCounter("Phase 3 - backtrace: ");
             Node<N> fin;
             fin.pos = coord_final;
             fin.set(res.g, res.f, 0);
             std::cout << "Final Score: " << fin << std::endl; // PAStarDistributedBacktrace.cpp:47
+            print_bound();
             std::vector<std::string> rows(N);
             for (int i = 0; i < N; i++) rows[i] = rowp[i];
             delete t;
@@ -488,7 +506,10 @@ class PAStar {
             js << "{\"finished\": " << res.finished << ", \"g\": " << res.g << ", \"f\": " << res.f << ", \"align_len\": " << res.align_len
                << ", \"rounds\": " << res.rounds << ", \"gpus\": " << gpus << ", \"search_ms\": " << res.kernel_ms
                << ", \"pair_tables_ms\": " << h->tables_ms << ", \"hash_type\": \"" << Coord<N>::get_hash_name() << "\", \"hash_shift\": "
-               << Coord<N>::get_hash_shift() << ", \"total\": ";
+               << Coord<N>::get_hash_shift();
+            if (options.weight_num)
+                js << ", \"weight\": " << std::setprecision(10) << (double)options.weight_num / wden << ", \"lower_bound\": " << lower_bound;
+            js << ", \"total\": ";
             one(res);
             js << ", \"partitions\": [";
             for (int i = 0; i < gpus; i++) {

@@ -1,7 +1,7 @@
 // pastar — drop-in CLI for the reference's ./bin/pastar (pastar/msa_pastar_main.cpp:56-193), GPU path.
 //
 //   pastar [-t N] [-s SHIFT] [-y FZORDER|FSUM|PZORDER|PSUM] [-v] [-h] [--memory_debug] file.fasta
-//   new, optional: [-g/--gpus N] [--batch K] [--table_capacity SLOTS] [--max_expansions E] [--metrics_json FILE]
+//   new, optional: [-g/--gpus N] [--batch K] [--table_capacity SLOTS] [--max_expansions E] [--metrics_json FILE] [--weight W]
 //
 // Same flags, exit codes (0 ok, 1 usage / not a regular file, -1 on exception) and stdout format as the reference
 // (phase timers, "Final Score:", "Similarity:", wrapped alignment, "Total nodes count:" table).  No MPI: the
@@ -61,6 +61,8 @@ static void usage(const char *argv0)
               << "  --table_capacity arg          closed/open table slots\n"
               << "  --max_expansions arg          stop after this many expansions\n"
               << "  --metrics_json arg            write the run's counters (total and per partition) as JSON\n"
+              << "  --weight arg                  bounded-suboptimal search: cost at most W (1..16) x the optimum,\n"
+              << "                                reported with a certified lower bound\n"
               << std::endl;
 }
 
@@ -82,7 +84,7 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
     };
     // Boost.ProgramOptions' default style lets a long option be shortened to any unambiguous prefix ("--thr 4", "--hash_t=FSUM")
     static const char *const long_names[] = {"version", "help", "memory_debug", "threads", "hash_shift", "hash_type", "gpus",
-                                             "batch", "table_capacity", "max_expansions", "metrics_json"};
+                                             "batch", "table_capacity", "max_expansions", "metrics_json", "weight"};
     auto canonical = [&](const std::string &arg) -> std::string {
         if (arg.size() < 3 || arg.compare(0, 2, "--") != 0) return arg;
         const size_t eq = arg.find('=');
@@ -117,6 +119,13 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
         else if (is_long(a, "table_capacity")) opt.table_capacity = std::stoll(value(i, a, "table_capacity"));
         else if (is_long(a, "max_expansions")) opt.max_expansions = std::stoll(value(i, a, "max_expansions"));
         else if (is_long(a, "metrics_json")) opt.metrics_json = value(i, a, "metrics_json");
+        else if (is_long(a, "weight")) {
+            const std::string v = value(i, a, "weight");
+            size_t used = 0;
+            const double w = std::stod(v, &used);
+            if (used != v.size() || !(w >= 1.0 && w <= 16.0)) throw std::invalid_argument("the argument for option '--weight' must be a number in 1..16");
+            opt.weight_num = (int)std::ceil(w * 1024.0); // weight num / 1024, rounded up
+        }
         else if (!a.empty() && a[0] == '-' && a.size() > 1) throw std::invalid_argument("unrecognised option '" + a + "'");
         else {
             filename = a; // file.fasta is position independent

@@ -242,6 +242,7 @@ extern "C" int pg_ctx_create(int n_seq, const char *const *seqs, const int *lens
         ctx->n_alpha = 0;
         for (bool b : seen) ctx->n_alpha += b ? 1 : 0;
     }
+    ctx->cost = hcost;
     PG_CUDA(ctx, cudaMalloc(&ctx->d_cost, sizeof(int32_t) * 8100));
     PG_CUDA(ctx, cudaMemcpy(ctx->d_cost, hcost.data(), sizeof(int32_t) * 8100, cudaMemcpyHostToDevice));
     dp.cost = ctx->d_cost;

@@ -73,9 +73,11 @@ struct ExpLane {
 // Stage the LUTs / HH table of one parent in the group's shared memory and compute the lane's B and E terms.
 // `sub` is the lane's index in the group and its low mask bits, `gmask` the shfl mask of the group's lanes.
 // s_grp points at GROUP_INTS ints of shared memory private to the group.
+// Weighted search (hnum > 1): every h term is floor(hnum * T * w / 2^hsh) instead of T * w, so the h sums are
+// h_w = sum over pairs of floor(weight * term), with h <= h_w <= weight * h (weight = hnum / 2^hsh >= 1).
 template <int N>
 __device__ __forceinline__ void pg_expand_prepare(const DevProblem &p, const PairMeta *meta, int *s_grp, const int (&pos)[N], int g,
-                                                  int parenti, int sub, unsigned gmask, ExpLane<N> &L)
+                                                  int parenti, int sub, unsigned gmask, ExpLane<N> &L, int hnum = 1, int hsh = 0)
 {
     using C = ExpCfg<N>;
     int *s_lutg = s_grp;
@@ -132,7 +134,7 @@ __device__ __forceinline__ void pg_expand_prepare(const DevProblem &p, const Pai
             const int gapc = ((parenti >> stays) & 1) ? p.gap_open : p.gap_ext;
             const int c = (dx & dy) ? cv[j] : ((dx | dy) ? gapc : p.gap_gap);
             s_lutg[e] = c * w;
-            s_luth[e] = tv[j] * w;
+            s_luth[e] = hnum > 1 ? (int)(((long long)tv[j] * w * hnum) >> hsh) : tv[j] * w;
         }
     }
     __syncwarp(gmask);

@@ -49,7 +49,7 @@ struct SearchCtrl {          // lives in device memory; mirrored to pinned host 
     int32_t plan_n;          // plan entries of the current round
     int32_t min_open_f;      // f of the first non-empty bucket after the last select (INT32_MAX if none)
     uint32_t chunk_bump;     // next free chunk
-    uint32_t pad0;
+    int32_t drop_lb;         // weighted search: min over dropped successors of a value <= their g + h (INT32_MAX if none)
     unsigned long long pops, expansions, generated, reopen, inserted, pushed, pruned, table_used; // table_used: records seen by insert kernels
     unsigned long long surv_n;   // local survivors of the current round (records in SearchState::d_surv)
     unsigned long long live_n;   // live parents of the current round (after the closed-bit claim)
@@ -66,6 +66,7 @@ struct pg_ctx {
     int len[PG_MAX_SEQ] = {0};
     std::vector<std::string> seqs;
     std::vector<PairGeom> pairs;
+    std::vector<int32_t> cost; // host copy of the 90 x 90 cost table (re-scoring of weighted-search alignments)
     DevProblem dp;
     uint8_t *d_seq = nullptr;
     int32_t *d_cost = nullptr;
@@ -82,6 +83,10 @@ struct pg_ctx {
     void *d_stage[2] = {nullptr, nullptr};
     size_t stage_bytes[2] = {0, 0};
     SearchState *search = nullptr;
+    // weighted search (pg_search_set_weight): f_w = g + h_w, h_w = sum of floor(wnum * term / 2^wsh); (1, 0) = exact A*
+    int wnum = 1, wsh = 0;
+    bool lb_valid = false;  // lower_bound holds the certified bound of the last pg_search / pg_multi_search
+    int32_t lower_bound = 0;
     // resident CTAs per SM of the kernels that opt in to > 48 KB of dynamic shared memory; 0 = attribute not set yet on
     // this context's device (N and the key width are fixed per context, so one slot per kernel / mode is enough)
     int occ_expand_batch = 0;
