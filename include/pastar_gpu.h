@@ -269,6 +269,34 @@ int pg_search_set_weight(pg_ctx *ctx, int32_t num, int32_t den);
  * bound, computed now (the driver takes the minimum over the partitions between rounds).  PG_ERR_STATE before any
  * search. */
 int pg_search_lower_bound(pg_ctx *ctx, int32_t *lower_bound);
+/* Cost of an alignment under the context's cost model (the arithmetic of the search's g; host code, O(cols * pairs)).
+ * rows: N NUL-terminated rows of exactly `cols` characters; each row with its '-' removed must spell the context's
+ * sequence and no column may hold gaps only.  PG_ERR_ARG with a message otherwise.  Needs no device. */
+int pg_score_alignment(pg_ctx *ctx, const char *const *rows, int32_t cols, int64_t *cost);
+/* Incumbent-bounded search - an opt-in extension of pg_search / pg_multi_search / pg_search_begin (the reference only
+ * searches from scratch; Ikeda & Imai 1999's "enhanced A*").  Scores `rows` (as pg_score_alignment), keeps a copy and
+ * makes its cost U the upper bound of every later search on the context: an exact search keeps only successors with
+ * g + h < U, a weighted one those with g + floor(h_w * floor(2^32 / weight) / 2^32) < U (a value <= g + h), and goals
+ * need g < U.  The bucket range, prune and goal limits and the value width follow from U.  Results:
+ *   finished = 1: a cheaper alignment, with its rows and cost;
+ *   finished = 2: the search ran out of nodes below U (or h(start) >= U): the incumbent's rows and g = U are returned,
+ *                 and an exact search then reports lower bound == U - a proof that the incumbent is optimal;
+ *   finished = 0: the expansion budget ran out (lower bound <= optimum <= U).
+ * The lower bound (pg_search_lower_bound) is also capped by U.  rows == NULL clears the incumbent.  PG_ERR_STATE while
+ * a step-wise search is active; pg_multi_search refuses contexts whose incumbent costs differ (PG_ERR_ARG). */
+int pg_search_set_incumbent(pg_ctx *ctx, const char *const *rows, int32_t cols);
+/* Anytime search on one GPU (restarting weighted A*, Richter, Thayer & Ruml, ICAPS 2010): phase k is a fresh pg_search
+ * at weight weight_num[k] / weight_den[k] (each as in pg_search_set_weight; n_phases in 1..64) whose incumbent is the
+ * best alignment so far - the caller's incumbent, if one is set, for phase 0.  cfg->max_expansions (0: none) is the
+ * budget over all phases.  The loop stops early once the best lower bound reaches the incumbent's cost, when a phase
+ * stops at the budget, or when a phase after the first runs out of table (PG_ERR_CAPACITY, kept as pg_last_error; the
+ * best alignment so far is returned).  res: counters summed over the phases, g and the rows (may be NULL) of the best alignment;
+ * finished = 1 when that alignment is proved optimal (lower bound == g), 2 when it is returned with a gap, 0 when no
+ * alignment is known.  phase_res / phase_lb (may be NULL): each phase's result and lower bound; phases that did not
+ * run are zeroed with phase_lb = -1.  Afterwards pg_search_lower_bound gives the maximum over the phases, the weight is
+ * what it was before the call and the incumbent is the alignment returned. */
+int pg_search_anytime(pg_ctx *ctx, const pg_search_config *cfg, const int32_t *weight_num, const int32_t *weight_den, int n_phases,
+                      pg_result *res, pg_result *phase_res, int32_t *phase_lb, char *const *rows);
 /* bytes per exchanged successor record for this context */
 int pg_xrec_stride(const pg_ctx *ctx);
 

@@ -10,6 +10,7 @@ Reference interface                                   -> here
   Node::getNeigh (Node.cpp:205-248)                    -> .expand_batch / .get_neigh
   PAStar::pa_star (PAStar.cpp:626-673)                 -> .search
   (no reference counterpart: bounded-suboptimal search) -> .search(weight=W) / .search_set_weight / .search_lower_bound
+  (no reference counterpart: incumbent / anytime search) -> .score_alignment / .search(incumbent=rows) / .anytime_search
 """
 import ctypes as C
 import math
@@ -111,6 +112,10 @@ def load_library():
         "pg_xrec_stride": ([vp], i32),
         "pg_search_set_weight": ([vp, C.c_int32, C.c_int32], i32),
         "pg_search_lower_bound": ([vp, C.POINTER(C.c_int32)], i32),
+        "pg_score_alignment": ([vp, C.POINTER(C.c_char_p), C.c_int32, C.POINTER(C.c_int64)], i32),
+        "pg_search_set_incumbent": ([vp, C.POINTER(C.c_char_p), C.c_int32], i32),
+        "pg_search_anytime": ([vp, C.POINTER(SearchConfig), C.POINTER(C.c_int32), C.POINTER(C.c_int32), i32, C.POINTER(Result),
+                               C.POINTER(Result), C.POINTER(C.c_int32), C.POINTER(C.c_char_p)], i32),
     }
     for name, (args, res) in sig.items():
         f = getattr(L, name)
@@ -125,7 +130,8 @@ EXPORTS = ["pg_release_cached_memory", "pg_search_note_rounds", "pg_search_set_d
            "pg_build_pair_tables", "pg_pair_table_shape", "pg_copy_pair_table", "pg_calculate_h", "pg_configure_hash",
            "pg_owner", "pg_expand_batch", "pg_expand_batch_dev", "pg_search", "pg_search_begin", "pg_search_round",
            "pg_search_outbox", "pg_search_insert_dev", "pg_search_status", "pg_search_lookup", "pg_search_end",
-           "pg_xrec_stride", "pg_search_set_weight", "pg_search_lower_bound"]
+           "pg_xrec_stride", "pg_search_set_weight", "pg_search_lower_bound", "pg_score_alignment", "pg_search_set_incumbent",
+           "pg_search_anytime"]
 
 WEIGHT_DEN = 1024
 
@@ -185,16 +191,21 @@ def bench_random_gather(nbytes, device=-1):
     return out.value
 
 
-def multi_search(gpus, table_capacity=0, batch_target=0, max_expansions=0, rounds_per_sync=0, want_rows=True, weight=1.0):
+def multi_search(gpus, table_capacity=0, batch_target=0, max_expansions=0, rounds_per_sync=0, want_rows=True, weight=1.0,
+                 incumbent=None):
     """pg_multi_search: one hash-owned partition per context in `gpus` (PastarGPU objects with their pair tables built and
     the same hash configuration; normally one per device, but contexts on one device work too), driven by this process.
     weight != 1: bounded-suboptimal search (see PastarGPU.search), set on every context.
+    incumbent (alignment rows): set on every context (see PastarGPU.search).
     Returns (total dict with lower_bound / weight_num / weight_den, list of per-partition dicts)."""
     L = load_library()
     g0 = gpus[0]
     if weight != 1.0:
         for g in gpus:
             g.search_set_weight(*weight_fraction(weight))
+    if incumbent is not None:
+        for g in gpus:
+            g.search_set_incumbent(incumbent)
     cfg = SearchConfig(len(gpus), 0, table_capacity, batch_target, max_expansions, rounds_per_sync, 0)
     res, parts = Result(), (Result * len(gpus))()
     handles = (C.c_void_p * len(gpus))(*[g.h for g in gpus])
@@ -406,18 +417,26 @@ class PastarGPU:
         return s[np.argsort(s["owner"], kind="stable")]
 
     # ---- (3)+(4) search
-    def search(self, table_capacity=0, batch_target=0, max_expansions=0, rounds_per_sync=0, want_rows=True, weight=1.0):
+    def _row_bufs(self, want_rows):
+        if not want_rows:
+            return None, None
+        total = sum(self.lens) + 1
+        bufs = [C.create_string_buffer(total) for _ in range(self.n)]
+        return (C.c_char_p * self.n)(*[C.cast(b, C.c_char_p) for b in bufs]), bufs
+
+    def search(self, table_capacity=0, batch_target=0, max_expansions=0, rounds_per_sync=0, want_rows=True, weight=1.0,
+               incumbent=None):
         """weight W > 1: bounded-suboptimal search (num / 1024 rounded up, as the CLI's --weight): g <= W x the optimum,
-        certified by the returned lower_bound (g * weight_den <= weight_num * lower_bound when finished)."""
+        certified by the returned lower_bound (g * weight_den <= weight_num * lower_bound when finished).
+        incumbent (alignment rows): set as the context's incumbent first (search_set_incumbent); finished == 2 then means
+        that nothing cheaper exists below its cost (its rows and cost are returned; an exact search proves it optimal)."""
         if weight != 1.0:
             self.search_set_weight(*weight_fraction(weight))
+        if incumbent is not None:
+            self.search_set_incumbent(incumbent)
         cfg = SearchConfig(1, 0, table_capacity, batch_target, max_expansions, rounds_per_sync, 0)
         res = Result()
-        rows, bufs = None, None
-        if want_rows:
-            total = sum(self.lens) + 1
-            bufs = [C.create_string_buffer(total) for _ in range(self.n)]
-            rows = (C.c_char_p * self.n)(*[C.cast(b, C.c_char_p) for b in bufs])
+        rows, bufs = self._row_bufs(want_rows)
         self._ck(self.L.pg_search(self.h, C.byref(cfg), C.byref(res), rows))
         d = res.as_dict()
         if want_rows and res.finished:
@@ -431,6 +450,52 @@ class PastarGPU:
         den <= num <= 16 den); (1, 1) is the exact search."""
         self._ck(self.L.pg_search_set_weight(self.h, int(num), int(den)))
         self.weight = (int(num), int(den))
+
+    def _rows_arg(self, rows):
+        bs = [r.encode() if isinstance(r, str) else bytes(r) for r in rows]
+        if len(bs) != self.n:
+            raise PastarError(1, "PG_ERR_ARG: %d alignment rows for %d sequences" % (len(bs), self.n))
+        return (C.c_char_p * self.n)(*bs), len(bs[0])
+
+    def score_alignment(self, rows):
+        """pg_score_alignment: the cost of an alignment (N rows of equal length, '-' for gaps) under this context's cost
+        model; PastarError PG_ERR_ARG if the rows do not align this context's sequences."""
+        arr, cols = self._rows_arg(rows)
+        v = C.c_int64()
+        self._ck(self.L.pg_score_alignment(self.h, arr, cols, C.byref(v)))
+        return v.value
+
+    def search_set_incumbent(self, rows):
+        """pg_search_set_incumbent: every later search keeps only what can beat this alignment's cost; None clears it."""
+        if rows is None:
+            self._ck(self.L.pg_search_set_incumbent(self.h, None, 0))
+        else:
+            arr, cols = self._rows_arg(rows)
+            self._ck(self.L.pg_search_set_incumbent(self.h, arr, cols))
+
+    def anytime_search(self, weights=(2, 1.25, 1), incumbent=None, table_capacity=0, batch_target=0, max_expansions=0,
+                       want_rows=True):
+        """pg_search_anytime: one fresh search per weight, each bounded by the best alignment so far (the incumbent, if
+        given, for the first); max_expansions is the budget over all phases.  Returns the usual dict (finished 1: proved
+        optimal, 2: an alignment with a gap to lower_bound, 0: none) with `lower_bound` and `phases`, one dict per phase
+        that ran: weight, g, lower_bound, expansions, finished."""
+        if incumbent is not None:
+            self.search_set_incumbent(incumbent)
+        fr = [weight_fraction(w) for w in weights]
+        k = len(fr)
+        nums = (C.c_int32 * k)(*[f[0] for f in fr])
+        dens = (C.c_int32 * k)(*[f[1] for f in fr])
+        cfg = SearchConfig(1, 0, table_capacity, batch_target, max_expansions, 0, 0)
+        res, pres, plb = Result(), (Result * k)(), (C.c_int32 * k)()
+        rows, bufs = self._row_bufs(want_rows)
+        self._ck(self.L.pg_search_anytime(self.h, C.byref(cfg), nums, dens, k, C.byref(res), pres, plb, rows))
+        d = res.as_dict()
+        if want_rows and res.finished:
+            d["rows"] = [b.value.decode() for b in bufs]
+        d["lower_bound"] = self.search_lower_bound()
+        d["phases"] = [{"weight": fr[i][0] / fr[i][1], "g": pres[i].g, "lower_bound": plb[i], "expansions": pres[i].expansions,
+                        "finished": pres[i].finished} for i in range(k) if plb[i] >= 0]
+        return d
 
     def search_lower_bound(self):
         """pg_search_lower_bound: certified lower bound on the optimal cost (of the last search, or of this partition of

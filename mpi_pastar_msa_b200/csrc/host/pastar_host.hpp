@@ -408,6 +408,9 @@ struct PAStarOpt { // PAStar.h:87-112, plus the GPU-side knobs (new, do not chan
     long long batch = 0, table_capacity = 0, max_expansions = 0;
     std::string metrics_json; // --metrics_json FILE: counters of the run as one JSON object (PAStarSyncData.cpp's gather, machine-readable)
     int weight_num = 0;       // --weight W: bounded-suboptimal search with weight weight_num / 1024 (0 = not given: exact search)
+    std::string incumbent;                  // --incumbent FILE: aligned FASTA of a known alignment (upper bound of the search)
+    std::vector<std::string> incumbent_rows; // its rows, checked against the input before any device call
+    std::vector<int32_t> anytime_num;        // --anytime W1,W2,...: one weighted phase per weight, num / 1024 (empty: not given)
 };
 
 int read_fasta_file(const std::string &name);
@@ -446,28 +449,53 @@ class PAStar {
         for (int i = 0; i < N; i++) rowp[i] = bufs[i].data();
         const int wden = 1024;
         int32_t lower_bound = 0;
+        const bool bounded = options.weight_num || !options.incumbent_rows.empty() || !options.anytime_num.empty();
+        std::vector<const char *> inc(N);
+        for (int i = 0; i < (int)options.incumbent_rows.size(); i++) inc[i] = options.incumbent_rows[i].c_str();
+        const int inc_cols = options.incumbent_rows.empty() ? 0 : (int)options.incumbent_rows[0].size();
+        int64_t inc_cost = 0;
+        const int n_phases = (int)options.anytime_num.size();
+        std::vector<pg_result> phase_res(n_phases);
+        std::vector<int32_t> phase_lb(n_phases, -1);
+        if (inc_cols) h->check(pg_score_alignment(h->ctx, inc.data(), inc_cols, &inc_cost), "pg_score_alignment");
         if (gpus == 1) {
             if (options.weight_num) h->check(pg_search_set_weight(h->ctx, options.weight_num, wden), "pg_search_set_weight");
+            if (inc_cols) h->check(pg_search_set_incumbent(h->ctx, inc.data(), inc_cols), "pg_search_set_incumbent");
             TimeCounter t("Phase 2: PA-Star running time: ");
-            h->check(pg_search(h->ctx, &cfg, &res, rowp.data()), "pg_search");
+            if (n_phases) {
+                const std::vector<int32_t> dens(n_phases, wden);
+                h->check(pg_search_anytime(h->ctx, &cfg, options.anytime_num.data(), dens.data(), n_phases, &res, phase_res.data(),
+                                           phase_lb.data(), rowp.data()),
+                         "pg_search_anytime");
+            } else {
+                h->check(pg_search(h->ctx, &cfg, &res, rowp.data()), "pg_search");
+            }
             parts[0] = res;
-            if (options.weight_num) h->check(pg_search_lower_bound(h->ctx, &lower_bound), "pg_search_lower_bound");
+            if (bounded) h->check(pg_search_lower_bound(h->ctx, &lower_bound), "pg_search_lower_bound");
         } else {
             // one hash-owned partition per GPU (the reference: one per thread x MPI rank, PAStar.cpp:107-117)
             std::vector<pg_ctx *> ctxs = h->contexts(gpus);
             for (pg_ctx *c : ctxs) h->check(pg_configure_hash(c, (int)options.hash_type, options.hash_shift), "pg_configure_hash");
             if (options.weight_num)
                 for (pg_ctx *c : ctxs) h->check(pg_search_set_weight(c, options.weight_num, wden), "pg_search_set_weight");
+            if (inc_cols)
+                for (pg_ctx *c : ctxs) h->check(pg_search_set_incumbent(c, inc.data(), inc_cols), "pg_search_set_incumbent");
             TimeCounter t("Phase 2: PA-Star running time: ");
             h->check(pg_multi_search(ctxs.data(), gpus, &cfg, &res, parts.data(), rowp.data()), "pg_multi_search");
-            if (options.weight_num) h->check(pg_search_lower_bound(ctxs[0], &lower_bound), "pg_search_lower_bound");
+            if (bounded) h->check(pg_search_lower_bound(ctxs[0], &lower_bound), "pg_search_lower_bound");
         }
-        // weighted search: the optimum is at least the lower bound, so g / bound is the certified ratio to it
+        // weighted, incumbent-bounded and anytime search: the optimum is at least the lower bound, so g / bound is the
+        // certified ratio to it (1: the alignment is proved optimal)
         auto print_bound = [&]() {
-            if (options.weight_num <= wden) return;
+            if (!(options.weight_num > wden || inc_cols || n_phases)) return;
             std::cout << "Lower bound: " << lower_bound;
             if (res.finished) std::cout << "\tg / lower bound: " << std::fixed << std::setprecision(4) << (double)res.g / lower_bound;
             std::cout << std::endl;
+            for (int k = 0; k < n_phases; k++)
+                if (phase_lb[k] >= 0)
+                    std::cout << "Anytime phase " << k + 1 << ": weight " << std::defaultfloat << std::setprecision(6) << (double)options.anytime_num[k] / wden
+                              << ", score " << phase_res[k].g << ", lower bound " << phase_lb[k] << ", expansions " << phase_res[k].expansions
+                              << std::endl;
         };
         if (!res.finished) {
             std::cout << "Search stopped at the expansion budget: " << res.expansions << " expansions, no alignment.\n";
@@ -508,7 +536,21 @@ class PAStar {
                << ", \"pair_tables_ms\": " << h->tables_ms << ", \"hash_type\": \"" << Coord<N>::get_hash_name() << "\", \"hash_shift\": "
                << Coord<N>::get_hash_shift();
             if (options.weight_num)
-                js << ", \"weight\": " << std::setprecision(10) << (double)options.weight_num / wden << ", \"lower_bound\": " << lower_bound;
+                js << ", \"weight\": " << std::setprecision(10) << (double)options.weight_num / wden;
+            if (bounded) js << ", \"lower_bound\": " << lower_bound;
+            if (inc_cols) js << ", \"incumbent\": " << inc_cost;
+            if (n_phases) {
+                js << ", \"phases\": [";
+                bool first = true;
+                for (int k = 0; k < n_phases; k++) {
+                    if (phase_lb[k] < 0) continue;
+                    js << (first ? "" : ", ") << "{\"weight\": " << std::setprecision(10) << (double)options.anytime_num[k] / wden
+                       << ", \"g\": " << phase_res[k].g << ", \"lower_bound\": " << phase_lb[k] << ", \"expansions\": "
+                       << phase_res[k].expansions << ", \"finished\": " << phase_res[k].finished << "}";
+                    first = false;
+                }
+                js << "]";
+            }
             js << ", \"total\": ";
             one(res);
             js << ", \"partitions\": [";

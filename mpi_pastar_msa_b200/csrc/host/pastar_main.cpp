@@ -2,11 +2,14 @@
 //
 //   pastar [-t N] [-s SHIFT] [-y FZORDER|FSUM|PZORDER|PSUM] [-v] [-h] [--memory_debug] file.fasta
 //   new, optional: [-g/--gpus N] [--batch K] [--table_capacity SLOTS] [--max_expansions E] [--metrics_json FILE] [--weight W]
+//                  [--incumbent FILE] [--anytime W1,W2,...]
 //
 // Same flags, exit codes (0 ok, 1 usage / not a regular file, -1 on exception) and stdout format as the reference
 // (phase timers, "Final Score:", "Similarity:", wrapped alignment, "Total nodes count:" table).  No MPI: the
 // reference's ranks x threads partitions map to GPUs of one box.
 #include "pastar_host.hpp"
+
+#include <algorithm>
 
 namespace pastar {
 
@@ -63,6 +66,10 @@ static void usage(const char *argv0)
               << "  --metrics_json arg            write the run's counters (total and per partition) as JSON\n"
               << "  --weight arg                  bounded-suboptimal search: cost at most W (1..16) x the optimum,\n"
               << "                                reported with a certified lower bound\n"
+              << "  --incumbent arg               aligned FASTA of a known alignment of the input: find a cheaper one or\n"
+              << "                                prove it optimal\n"
+              << "  --anytime arg                 comma-separated weights (1..16), one search per weight, each bounded\n"
+              << "                                by the best alignment so far (one GPU)\n"
               << std::endl;
 }
 
@@ -84,7 +91,8 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
     };
     // Boost.ProgramOptions' default style lets a long option be shortened to any unambiguous prefix ("--thr 4", "--hash_t=FSUM")
     static const char *const long_names[] = {"version", "help", "memory_debug", "threads", "hash_shift", "hash_type", "gpus",
-                                             "batch", "table_capacity", "max_expansions", "metrics_json", "weight"};
+                                             "batch", "table_capacity", "max_expansions", "metrics_json", "weight",
+                                             "incumbent", "anytime"};
     auto canonical = [&](const std::string &arg) -> std::string {
         if (arg.size() < 3 || arg.compare(0, 2, "--") != 0) return arg;
         const size_t eq = arg.find('=');
@@ -106,6 +114,13 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
         const std::string ll = std::string("--") + l;
         return a == ll || a.compare(0, ll.size() + 1, ll + "=") == 0;
     };
+    auto weight_num = [](const std::string &v, const char *longname) { // W in 1..16 as num / 1024, rounded up
+        size_t used = 0;
+        const double w = std::stod(v, &used);
+        if (used != v.size() || !(w >= 1.0 && w <= 16.0))
+            throw std::invalid_argument(std::string("the argument for option '--") + longname + "' must be a number in 1..16");
+        return (int)std::ceil(w * 1024.0);
+    };
     for (int i = 1; i < argc; i++) {
         const std::string a = canonical(argv[i]);
         if (a == "-v" || a == "--version") version = true;
@@ -119,12 +134,18 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
         else if (is_long(a, "table_capacity")) opt.table_capacity = std::stoll(value(i, a, "table_capacity"));
         else if (is_long(a, "max_expansions")) opt.max_expansions = std::stoll(value(i, a, "max_expansions"));
         else if (is_long(a, "metrics_json")) opt.metrics_json = value(i, a, "metrics_json");
-        else if (is_long(a, "weight")) {
-            const std::string v = value(i, a, "weight");
-            size_t used = 0;
-            const double w = std::stod(v, &used);
-            if (used != v.size() || !(w >= 1.0 && w <= 16.0)) throw std::invalid_argument("the argument for option '--weight' must be a number in 1..16");
-            opt.weight_num = (int)std::ceil(w * 1024.0); // weight num / 1024, rounded up
+        else if (is_long(a, "weight")) opt.weight_num = weight_num(value(i, a, "weight"), "weight");
+        else if (is_long(a, "incumbent")) opt.incumbent = value(i, a, "incumbent");
+        else if (is_long(a, "anytime")) {
+            const std::string v = value(i, a, "anytime");
+            opt.anytime_num.clear();
+            for (size_t at = 0;;) {
+                const size_t comma = v.find(',', at);
+                opt.anytime_num.push_back(weight_num(v.substr(at, comma == std::string::npos ? std::string::npos : comma - at), "anytime"));
+                if (comma == std::string::npos) break;
+                at = comma + 1;
+            }
+            if (opt.anytime_num.size() > 64) throw std::invalid_argument("the argument for option '--anytime' has more than 64 weights");
         }
         else if (!a.empty() && a[0] == '-' && a.size() > 1) throw std::invalid_argument("unrecognised option '" + a + "'");
         else {
@@ -137,6 +158,8 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
     else if (hash_read == "PZORDER") opt.hash_type = HashPZorder;
     else if (hash_read == "PSUM") opt.hash_type = HashPSum;
     else throw std::invalid_argument("the argument for option '--hash_type' is invalid");
+    if (!opt.anytime_num.empty() && opt.weight_num) throw std::invalid_argument("option '--anytime' cannot be combined with '--weight'");
+    if (!opt.anytime_num.empty() && opt.gpus != 1) throw std::invalid_argument("option '--anytime' runs on one GPU (--gpus 1)");
     if (version) {
         std::cout << "msa_pastar, version 1.0\n";
         std::exit(0);
@@ -201,6 +224,43 @@ void print_alignment(const std::vector<std::string> &rows) // backtrace.cpp:171-
     }
 }
 
+// --incumbent FILE: an aligned FASTA (records as read_fasta_file reads them, '-' for gaps) with the input's records in
+// the input's order.  Checked here, before any device call: the rows must be of equal length, spell the input sequences
+// once their gaps are removed, and hold no column of gaps only.  Returns an empty string or what is wrong.
+static std::string read_incumbent(const std::string &name, std::vector<std::string> &rows)
+{
+    struct stat st;
+    if (stat(name.c_str(), &st) != 0 || !S_ISREG(st.st_mode)) return "not a regular file";
+    std::ifstream file(name.c_str());
+    if (!file.is_open()) return "cannot be opened";
+    rows.clear();
+    std::string cur, buf;
+    while (getline(file, buf)) {
+        if (!buf.empty() && buf.back() == '\r') buf.pop_back();
+        if (buf.empty() || buf[0] == '>') {
+            if (!cur.empty()) rows.push_back(cur);
+            cur.clear();
+        } else {
+            cur += buf;
+        }
+    }
+    if (!cur.empty()) rows.push_back(cur);
+    const int n = Sequences::get_seq_num();
+    if ((int)rows.size() != n) return std::to_string(rows.size()) + " records for " + std::to_string(n) + " input sequences";
+    for (int i = 0; i < n; i++) {
+        if (rows[i].size() != rows[0].size()) return "record " + std::to_string(i + 1) + " differs in length from record 1";
+        std::string r = rows[i];
+        r.erase(std::remove(r.begin(), r.end(), '-'), r.end());
+        if (r != Sequences::getInstance()->get_seq(i)) return "record " + std::to_string(i + 1) + " does not spell input sequence " + std::to_string(i + 1);
+    }
+    for (size_t c = 0; c < rows[0].size(); c++) {
+        bool gaps = true;
+        for (int i = 0; i < n && gaps; i++) gaps = rows[i][c] == '-';
+        if (gaps) return "column " + std::to_string(c + 1) + " holds gaps only";
+    }
+    return "";
+}
+
 static int pa_star_run_core(const PAStarOpt &opt) // msa_pastar_main.cpp:20-37
 {
     HeuristicHPair::getInstance()->init();
@@ -247,6 +307,13 @@ int main(int argc, char *argv[])
     opt.mpiMax = opt.threads_num;
     opt.totalThreads = opt.mpiCommSize * opt.threads_num;
     if (read_fasta_file(filename) != 0) return 1;
+    if (!opt.incumbent.empty()) {
+        const std::string why = read_incumbent(opt.incumbent, opt.incumbent_rows);
+        if (!why.empty()) {
+            std::cerr << "Fatal error: --incumbent " << opt.incumbent << ": " << why << std::endl;
+            return 1;
+        }
+    }
     const int ret = pa_star_run(opt);
     HeuristicHPair::getInstance()->destroyInstance();
     return ret;

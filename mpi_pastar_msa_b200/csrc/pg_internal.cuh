@@ -87,6 +87,10 @@ struct pg_ctx {
     int wnum = 1, wsh = 0;
     bool lb_valid = false;  // lower_bound holds the certified bound of the last pg_search / pg_multi_search
     int32_t lower_bound = 0;
+    // incumbent (pg_search_set_incumbent): a known alignment and its cost U; every later search keeps only what can beat
+    // U.  inc_cost < 0: none
+    std::vector<std::string> inc_rows;
+    long long inc_cost = -1;
     // resident CTAs per SM of the kernels that opt in to > 48 KB of dynamic shared memory; 0 = attribute not set yet on
     // this context's device (N and the key width are fixed per context, so one slot per kernel / mode is enough)
     int occ_expand_batch = 0;

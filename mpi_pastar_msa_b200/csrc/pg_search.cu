@@ -103,6 +103,7 @@ struct SearchState {
     int64_t batch_target = 0;
     int f0 = 0, f_range = 0, ub = 0;
     int goal_limit = 0;      // goals with g >= this are dropped (the all-advance cost + 1); weighted: every successor
+    long long inc = LLONG_MAX; // the incumbent's cost U when the search began (LLONG_MAX: none)
     // multi-partition outboxes
     char *d_outbox = nullptr;
     unsigned long long *d_outbox_count = nullptr;
@@ -266,10 +267,13 @@ struct DevSearch {
     int f0, f_range;              // bucket 0 is f == f0; number of buckets
     // weighted search (pg_search_set_weight): h terms are floor(hnum * term >> hsh); hnum == 1: exact A*.  hrecip =
     // floor(2^32 / weight) turns a dropped successor's h_w back into a value <= its h.  goal_limit: goals (and, weighted,
-    // every successor) with g >= this are dropped - the all-advance cost + 1.
+    // every successor) with g >= this are dropped - the all-advance cost + 1.  inc_limit: the incumbent's cost U
+    // (INT_MAX without one); a weighted successor is dropped when its lower bound g + floor(h_w * hrecip / 2^32) <= g + h
+    // reaches it.  The exact search carries U in prune_limit and goal_limit alone.
     int hnum, hsh;
     unsigned hrecip;
     int goal_limit;
+    int inc_limit;
     unsigned long long *live;     // compacted live parents of the round, word-major: live[w * live_cap + i]
     unsigned long long live_cap;
     unsigned long long *surv;     // local survivors of the round
@@ -1397,10 +1401,12 @@ __global__ void __launch_bounds__(256, PG_EXPAND_CTAS) expand_probe_kernel(const
                             if (!drop) atomicMin(&c->best_goal, gn);
                         } else if (d.hnum > 1) {
                             // weighted: f_w no longer bounds g, so g beyond the all-advance cost is dropped as well; what
-                            // the f_w test drops may still lie on an optimal path - its g + h is kept for the lower bound
-                            drop = drop || gn >= d.goal_limit;
+                            // the f_w test drops may still lie on an optimal path - its g + h is kept for the lower bound.
+                            // With an incumbent, a successor whose bound reaches its cost U cannot lead to a cheaper one.
+                            const int lbn = gn + (int)(((unsigned long long)(unsigned)(fn - gn) * d.hrecip) >> 32);
+                            drop = drop || gn >= d.goal_limit || lbn >= d.inc_limit;
                             if (drop)
-                                s_droplb[threadIdx.x] = min(s_droplb[threadIdx.x], gn + (int)(((unsigned long long)(unsigned)(fn - gn) * d.hrecip) >> 32));
+                                s_droplb[threadIdx.x] = min(s_droplb[threadIdx.x], lbn);
                         }
                         if (drop) {
                             n_pruned++;
@@ -2027,6 +2033,7 @@ DevSearch dev_search(const pg_ctx *ctx)
     d.hsh = ctx->wsh;
     d.hrecip = ctx->wnum > 1 ? (unsigned)((1ull << (32 + ctx->wsh)) / (unsigned long long)ctx->wnum) : 0u; // floor(2^32 / weight) < 2^32
     d.goal_limit = s->goal_limit;
+    d.inc_limit = (int)std::min<long long>(s->inc, INT_MAX);
     d.live_cap = s->live_cap;
     d.surv = s->d_surv;
     d.surv_cap = s->surv_cap;
@@ -2476,17 +2483,24 @@ extern "C" int pg_search_begin(pg_ctx *ctx, const pg_search_config *cfg)
     const long long wub = ((long long)s->ub * ctx->wnum) >> ctx->wsh;
     if (wub >= INT_MAX)
         return pg_fail(ctx, PG_ERR_UNSUPPORTED, "weight x upper bound does not fit 32 bits");
-    long long range = wub - s->f0 + 2;
+    // incumbent of cost U: only what can beat U is kept - exact: f < U; weighted: g < U, f_w <= floor(weight * U) - so the
+    // bucket range, the prune and goal limits and the value width shrink with U.  They carry the whole bound of the exact
+    // search; the weighted one also drops successors by their lower bound (DevSearch::inc_limit).
+    s->inc = ctx->inc_cost >= 0 ? ctx->inc_cost : LLONG_MAX;
+    const long long winc = s->inc == LLONG_MAX ? LLONG_MAX : (s->inc * ctx->wnum) >> ctx->wsh;
+    const long long f_end = std::min(wub, winc);                                 // last bucket's f
+    const long long f_lim = ctx->wnum > 1 ? f_end + 1 : std::min(wub + 1, s->inc); // successors with f >= this are dropped
+    long long range = f_end - s->f0 + 2;
     if (range < 2) range = 2;
     if (range > (1ll << 27)) // 1 GiB of bucket heads at most: a wider f range is refused, never clamped
         return pg_fail(ctx, PG_ERR_UNSUPPORTED, "f range (weight x upper bound - h(start)) exceeds 2^27 open-list buckets");
     s->f_range = (int)range;
-    s->goal_limit = (int)std::min<long long>((long long)s->ub + 1, (long long)s->f0 + s->f_range);
+    s->goal_limit = (int)std::min(std::min((long long)s->ub + 1, s->inc), (long long)s->f0 + s->f_range);
 
     // ---- value width: 4 bytes when g (<= the upper bound), the open bit and the move mask fit 32 bits
     {
         const char *fv = getenv("PG_VALW"); // PG_VALW=8 forces the wide form (tests)
-        const bool fits = s->keyw == 1 && (unsigned long long)s->ub + 2ull < (1ull << (31 - ctx->n));
+        const bool fits = s->keyw == 1 && (unsigned long long)std::min((long long)s->ub, s->inc - 1) + 2ull < (1ull << (31 - ctx->n));
         s->valw = (fits && !(fv && atoi(fv) == 8)) ? 4 : 8;
         s->nb = s->valw == 4 ? ctx->n : 31;
         s->gs = s->nb + 1;
@@ -2600,7 +2614,7 @@ extern "C" int pg_search_begin(pg_ctx *ctx, const pg_search_config *cfg)
     c.f_range = s->f_range;
     c.cursor = 0;
     c.best_goal = INT_MAX;
-    c.prune_limit = (int)std::min<long long>(wub + 1, (long long)s->f0 + s->f_range);
+    c.prune_limit = (int)std::min(f_lim, (long long)s->f0 + s->f_range);
     c.min_open_f = s->f0;
     c.drop_lb = INT_MAX;
     PG_CUDA(ctx, cudaMemcpyAsync(s->d_ctrl, &c, sizeof(c), cudaMemcpyHostToDevice, ctx->stream));
@@ -2886,12 +2900,13 @@ int census_ctx(pg_ctx *ctx, int64_t *open_size, int64_t *closed_size, long long 
 
 // Lower bound on the optimal cost from this partition's state (the control block read at the last sync, no records in
 // flight): min of (a) g + h over the open entries, (b) the dropped successors' bound (weighted search only), (c) the best
-// goal and (d) the all-advance cost.  The first node of an optimal path that is not closed with its optimal g is open
-// with that g or was dropped, so the minimum is at most the optimum.
+// goal, (d) the all-advance cost and (e) the incumbent's cost U.  The first node of an optimal path that is not closed
+// with its optimal g is open with that g or was dropped, so the minimum is at most the optimum.  Successors dropped for
+// the incumbent have g + h >= U, and U >= the optimum since U is the cost of an alignment.
 long long partition_lb(const SearchState *s, long long open_lb)
 {
     const SearchCtrl *c = s->h_ctrl;
-    return std::min(std::min(open_lb, (long long)s->ub), std::min((long long)c->drop_lb, (long long)c->best_goal));
+    return std::min(std::min(std::min(open_lb, (long long)s->ub), std::min((long long)c->drop_lb, (long long)c->best_goal)), s->inc);
 }
 
 // g of the alignment spelled by `masks` (origin first) under the context's cost model (ub_kernel's arithmetic,
@@ -2922,7 +2937,72 @@ long long rescore_masks(const pg_ctx *ctx, const std::vector<uint32_t> &masks)
     }
     return sum;
 }
+
+// Move masks (origin first) of the alignment `rows`: N NUL-terminated rows of `cols` characters each, every row with its
+// '-' removed spelling the context's sequence, no column of gaps only.  PG_ERR_ARG with a message otherwise.
+int alignment_masks(pg_ctx *ctx, const char *const *rows, int32_t cols, std::vector<uint32_t> &masks)
+{
+    if (cols < 1) return pg_fail(ctx, PG_ERR_ARG, "alignment: cols must be positive");
+    masks.assign((size_t)cols, 0u);
+    for (int i = 0; i < ctx->n; i++) {
+        const char *r = rows[i];
+        if (!r) return pg_fail(ctx, PG_ERR_ARG, "alignment: row " + std::to_string(i) + " is NULL");
+        int at = 0;
+        for (int c = 0; c < cols; c++) {
+            if (r[c] == 0) return pg_fail(ctx, PG_ERR_ARG, "alignment: row " + std::to_string(i) + " is shorter than cols");
+            if (r[c] == '-') continue;
+            if (at >= ctx->len[i] || r[c] != ctx->seqs[i][at])
+                return pg_fail(ctx, PG_ERR_ARG, "alignment: row " + std::to_string(i) + " does not spell sequence " + std::to_string(i));
+            at++;
+            masks[c] |= 1u << i;
+        }
+        if (r[cols] != 0) return pg_fail(ctx, PG_ERR_ARG, "alignment: row " + std::to_string(i) + " is longer than cols");
+        if (at != ctx->len[i])
+            return pg_fail(ctx, PG_ERR_ARG, "alignment: row " + std::to_string(i) + " does not spell sequence " + std::to_string(i));
+    }
+    for (int c = 0; c < cols; c++)
+        if (masks[c] == 0) return pg_fail(ctx, PG_ERR_ARG, "alignment: column " + std::to_string(c) + " holds gaps only");
+    return PG_OK;
+}
+
+// The incumbent as a search result: g = f = U, its rows when the caller wants them.
+void emit_incumbent(const pg_ctx *ctx, pg_result *res, char *const *rows)
+{
+    res->g = res->f = (int32_t)ctx->inc_cost;
+    res->align_len = (int32_t)ctx->inc_rows[0].size();
+    if (rows)
+        for (int i = 0; i < ctx->n; i++) memcpy(rows[i], ctx->inc_rows[i].c_str(), ctx->inc_rows[i].size() + 1);
+}
 } // namespace
+
+extern "C" int pg_score_alignment(pg_ctx *ctx, const char *const *rows, int32_t cols, int64_t *cost)
+{
+    if (!ctx || !rows || !cost) return PG_ERR_ARG;
+    std::vector<uint32_t> masks;
+    const int rc = alignment_masks(ctx, rows, cols, masks);
+    if (rc != PG_OK) return rc;
+    *cost = (int64_t)rescore_masks(ctx, masks);
+    return PG_OK;
+}
+
+extern "C" int pg_search_set_incumbent(pg_ctx *ctx, const char *const *rows, int32_t cols)
+{
+    if (!ctx) return PG_ERR_ARG;
+    if (ctx->search && ctx->search->active && ctx->search->stepwise)
+        return pg_fail(ctx, PG_ERR_STATE, "pg_search_set_incumbent: a step-wise search is active (pg_search_end first)");
+    if (!rows) {
+        ctx->inc_rows.clear();
+        ctx->inc_cost = -1;
+        return PG_OK;
+    }
+    int64_t cost = 0;
+    const int rc = pg_score_alignment(ctx, rows, cols, &cost);
+    if (rc != PG_OK) return rc;
+    if (cost < 0 || cost >= INT_MAX) return pg_fail(ctx, PG_ERR_ARG, "pg_search_set_incumbent: the alignment's cost is outside 0..2^31-2");
+    ctx->inc_rows.assign(rows, rows + ctx->n);
+    ctx->inc_cost = cost;
+    return PG_OK;
+}
 
 extern "C" int pg_search(pg_ctx *ctx, const pg_search_config *cfg_in, pg_result *res, char *const *rows)
 {
@@ -2949,7 +3029,10 @@ extern "C" int pg_search(pg_ctx *ctx, const pg_search_config *cfg_in, pg_result 
     cudaGraph_t graph = nullptr;
     cudaGraphExec_t gexec = nullptr;
     bool try_graph = !s->profile && !getenv("PG_NO_GRAPH");
-    for (long group = 0;; group++) {
+    // h(start) >= U: no alignment is cheaper than the incumbent, and no round needs to run to know it
+    const bool at_once = s->f0 >= s->inc;
+    if (at_once) rc = sync_ctrl(ctx);
+    for (long group = 0; !at_once; group++) {
         if (gexec) {
             PG_CUDA(ctx, cudaGraphLaunch(gexec, ctx->stream));
             s->rounds += per_sync;
@@ -2996,13 +3079,17 @@ extern "C" int pg_search(pg_ctx *ctx, const pg_search_config *cfg_in, pg_result 
     s->kernel_ms = ms;
     fill_counters(s, res);
     res->finished = s->h_ctrl->done == 1 ? 1 : 0;
+    if (s->inc != LLONG_MAX && (at_once || s->h_ctrl->done == 2)) // exhausted below U: the incumbent stands
+        res->finished = 2;
 
     // ---- open / closed census (the reference's final report, PAStar.cpp:591-619) and the search's lower bound
     long long open_lb = 0;
     if ((rc = census_ctx(ctx, &res->open_size, &res->closed_size, &open_lb)) != PG_OK) return rc;
     const long long lb = partition_lb(s, open_lb);
 
-    if (res->finished) {
+    if (res->finished == 2) {
+        emit_incumbent(ctx, res, rows);
+    } else if (res->finished) {
         res->g = res->f = s->h_ctrl->best_goal; // h(goal) = 0
         int total = 0;
         for (int i = 0; i < ctx->n; i++) total += ctx->len[i];
@@ -3078,6 +3165,92 @@ extern "C" int pg_search_lower_bound(pg_ctx *ctx, int32_t *lower_bound)
     return PG_OK;
 }
 
+extern "C" int pg_search_anytime(pg_ctx *ctx, const pg_search_config *cfg_in, const int32_t *weight_num, const int32_t *weight_den,
+                                 int n_phases, pg_result *res, pg_result *phase_res, int32_t *phase_lb, char *const *rows)
+{
+    if (!ctx || !res || !weight_num || !weight_den) return PG_ERR_ARG;
+    if (n_phases < 1 || n_phases > 64) return pg_fail(ctx, PG_ERR_ARG, "pg_search_anytime: n_phases must be in 1..64");
+    for (int k = 0; k < n_phases; k++) {
+        const int32_t num = weight_num[k], den = weight_den[k];
+        if (den < 1 || den > 1024 || (den & (den - 1)) != 0 || num < den || num > 16 * den)
+            return pg_fail(ctx, PG_ERR_ARG, "pg_search_anytime: phase " + std::to_string(k) + ": den must be a power of two in 1..1024 and den <= num <= 16 den");
+    }
+    if (ctx->search && ctx->search->active && ctx->search->stepwise)
+        return pg_fail(ctx, PG_ERR_STATE, "pg_search_anytime: a step-wise search is active (pg_search_end first)");
+    pg_search_config cfg;
+    if (cfg_in)
+        cfg = *cfg_in;
+    else
+        memset(&cfg, 0, sizeof(cfg));
+    memset(res, 0, sizeof(*res));
+    res->g = res->f = -1;
+    for (int k = 0; k < n_phases; k++) {
+        if (phase_res) memset(&phase_res[k], 0, sizeof(pg_result));
+        if (phase_lb) phase_lb[k] = -1;
+    }
+    const auto t0 = std::chrono::steady_clock::now();
+    const int wnum0 = ctx->wnum, wsh0 = ctx->wsh;
+    size_t total = 1;
+    for (int i = 0; i < ctx->n; i++) total += (size_t)ctx->len[i];
+    std::vector<std::vector<char>> bufs(ctx->n, std::vector<char>(total));
+    std::vector<char *> rowp(ctx->n);
+    for (int i = 0; i < ctx->n; i++) rowp[i] = bufs[i].data();
+    bool any = false;
+    long long lb = 0; // the maximum over the phases of their certified bounds
+    int rc = PG_OK;
+    for (int k = 0; k < n_phases; k++) {
+        if (any && ctx->inc_cost >= 0 && lb >= ctx->inc_cost) break; // the incumbent is proved optimal
+        pg_search_config pc = cfg;
+        if (cfg.max_expansions > 0) {
+            if (res->expansions >= cfg.max_expansions) break;
+            pc.max_expansions = cfg.max_expansions - res->expansions;
+        }
+        if ((rc = pg_search_set_weight(ctx, weight_num[k], weight_den[k])) != PG_OK) break;
+        pg_result pr;
+        if ((rc = pg_search(ctx, &pc, &pr, rowp.data())) != PG_OK) {
+            // a phase that runs out of table ends the loop as the budget does: a lower weight keeps more nodes, so the
+            // later phases would too.  The best alignment so far stands (pg_last_error says why the loop stopped).
+            if (rc == PG_ERR_CAPACITY && any) rc = PG_OK;
+            break;
+        }
+        // a phase that finishes found an alignment cheaper than the incumbent: it is the next phase's incumbent
+        if (pr.finished == 1 && (rc = pg_search_set_incumbent(ctx, rowp.data(), pr.align_len)) != PG_OK) break;
+        lb = any ? std::max(lb, (long long)ctx->lower_bound) : (long long)ctx->lower_bound;
+        any = true;
+        if (phase_res) phase_res[k] = pr;
+        if (phase_lb) phase_lb[k] = ctx->lower_bound;
+        res->pops += pr.pops;
+        res->expansions += pr.expansions;
+        res->generated += pr.generated;
+        res->reopen += pr.reopen;
+        res->open_size += pr.open_size;
+        res->closed_size += pr.closed_size;
+        res->rounds += pr.rounds;
+        res->probed += pr.probed;
+        res->pushed += pr.pushed;
+        res->inserted += pr.inserted;
+        res->survivors += pr.survivors;
+        res->kernel_ms += pr.kernel_ms;
+        res->expand_ms += pr.expand_ms;
+        res->select_ms += pr.select_ms;
+        res->claim_ms += pr.claim_ms;
+        res->insert_ms += pr.insert_ms;
+        res->inbox_ms += pr.inbox_ms;
+        if (pr.finished == 0) break; // the expansion budget is spent
+    }
+    ctx->wnum = wnum0;
+    ctx->wsh = wsh0;
+    if (rc != PG_OK) return rc;
+    if (ctx->inc_cost >= 0) {
+        emit_incumbent(ctx, res, rows);
+        res->finished = any && lb >= ctx->inc_cost ? 1 : 2;
+    }
+    ctx->lower_bound = (int32_t)lb;
+    ctx->lb_valid = any;
+    res->seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+    return PG_OK;
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // pg_multi_search: the hash-partitioned search over G GPUs of one box, driven by ONE host process (the pastar CLI).
 // Replaces PAStar<N>::pa_star with threads x MPI ranks (PAStar.cpp:626-673) plus sender / receiver / decoder threads
@@ -3096,6 +3269,9 @@ extern "C" int pg_multi_search(pg_ctx *const *ctxs, int n_gpus, const pg_search_
     for (int i = 1; i < n_gpus; i++)
         if (ctxs[i]->wnum != c0->wnum || ctxs[i]->wsh != c0->wsh)
             return pg_fail(c0, PG_ERR_ARG, "pg_multi_search: the contexts' search weights differ (pg_search_set_weight)");
+    for (int i = 1; i < n_gpus; i++)
+        if (ctxs[i]->inc_cost != c0->inc_cost)
+            return pg_fail(c0, PG_ERR_ARG, "pg_multi_search: the contexts' incumbent costs differ (pg_search_set_incumbent)");
     if (n_gpus == 1) {
         int rc = pg_search(c0, cfg_in, total, rows);
         if (rc == PG_OK && parts) parts[0] = *total;
@@ -3197,13 +3373,16 @@ extern "C" int pg_multi_search(pg_ctx *const *ctxs, int n_gpus, const pg_search_
     const int per_sync = cfg.rounds_per_sync > 0 ? cfg.rounds_per_sync : (stamped ? 8 : 4);
     int best = INT_MAX, min_open = INT_MAX;
     bool finished = false;
+    // every partition empty with no goal below the incumbent's cost U (or h(start) >= U, when no round runs): it stands
+    const long long inc = c0->search->inc;
+    bool exhausted = c0->search->f0 >= inc;
     std::vector<pg_result> pr(G);
     std::vector<cudaEvent_t> ev2(G, nullptr); // second event per device: rounds alternate, so a peer one round ahead does not re-record the one being waited for
     for (int i = 0; i < G; i++) {
         MG_CUDA(i, cudaSetDevice(ctxs[i]->device));
         MG_CUDA(i, cudaEventCreateWithFlags(&ev2[i], cudaEventDisableTiming));
     }
-    {
+    if (!exhausted) {
         std::atomic<int> fail(-1), arrive(0), gsense(0), stop(0);
         std::vector<std::atomic<long>> recorded(G);
         for (auto &r : recorded) r.store(-1);
@@ -3316,6 +3495,7 @@ extern "C" int pg_multi_search(pg_ctx *const *ctxs, int n_gpus, const pg_search_
                     min_open = mo;
                     if (mo >= bs || mo == INT_MAX) {
                         finished = bs != INT_MAX;
+                        exhausted = !finished && inc != LLONG_MAX;
                         stop.store(1);
                     } else if (cfg.max_expansions > 0 && expansions >= cfg.max_expansions) {
                         stop.store(1);
@@ -3344,6 +3524,12 @@ extern "C" int pg_multi_search(pg_ctx *const *ctxs, int n_gpus, const pg_search_
             cleanup();
             return rc;
         }
+    } else {
+        for (int i = 0; i < G; i++) {
+            cudaSetDevice(ctxs[i]->device);
+            if (ev2[i]) cudaEventDestroy(ev2[i]);
+        }
+        for (int i = 0; i < G; i++) MG_CHECK(i, pg_search_status(ctxs[i], nullptr, nullptr, &pr[i]));
     }
 
     // ---- results: counters per partition and summed; open / closed census (PAStar.cpp:591-619); the lower bound is the
@@ -3367,8 +3553,11 @@ extern "C" int pg_multi_search(pg_ctx *const *ctxs, int n_gpus, const pg_search_
         total->rounds = pr[i].rounds;
         if (parts) parts[i] = pr[i];
     }
-    total->finished = finished ? 1 : 0;
-    if (finished) {
+    total->finished = finished ? 1 : (exhausted ? 2 : 0);
+    if (exhausted) {
+        for (int i = 0; i < G; i++) pr[i].finished = 2;
+        emit_incumbent(c0, total, rows);
+    } else if (finished) {
         total->g = total->f = best;
         // distributed backtrace (PAStarDistributedBacktrace.cpp:18-214): the owner of each coordinate answers
         const int n = c0->n;
