@@ -209,16 +209,9 @@ def multi_search(gpus, table_capacity=0, batch_target=0, max_expansions=0, round
     cfg = SearchConfig(len(gpus), 0, table_capacity, batch_target, max_expansions, rounds_per_sync, 0)
     res, parts = Result(), (Result * len(gpus))()
     handles = (C.c_void_p * len(gpus))(*[g.h for g in gpus])
-    rows, bufs = None, None
-    if want_rows:
-        total = sum(g0.lens) + 1
-        bufs = [C.create_string_buffer(total) for _ in range(g0.n)]
-        rows = (C.c_char_p * g0.n)(*[C.cast(b, C.c_char_p) for b in bufs])
+    rows, bufs = g0._row_bufs(want_rows)
     g0._ck(L.pg_multi_search(handles, len(gpus), C.byref(cfg), C.byref(res), parts, rows))
-    d = res.as_dict()
-    if want_rows and res.finished:
-        d["rows"] = [b.value.decode() for b in bufs]
-    d["lower_bound"] = g0.search_lower_bound()
+    d = g0._result(res, bufs)
     d["weight_num"], d["weight_den"] = g0.weight
     return d, [p.as_dict() for p in parts]
 
@@ -424,6 +417,14 @@ class PastarGPU:
         bufs = [C.create_string_buffer(total) for _ in range(self.n)]
         return (C.c_char_p * self.n)(*[C.cast(b, C.c_char_p) for b in bufs]), bufs
 
+    def _result(self, res, bufs):
+        """A search's Result as a dict, with the rows found (when _row_bufs gave buffers) and the certified lower bound."""
+        d = res.as_dict()
+        if bufs is not None and res.finished:
+            d["rows"] = [b.value.decode() for b in bufs]
+        d["lower_bound"] = self.search_lower_bound()
+        return d
+
     def search(self, table_capacity=0, batch_target=0, max_expansions=0, rounds_per_sync=0, want_rows=True, weight=1.0,
                incumbent=None):
         """weight W > 1: bounded-suboptimal search (num / 1024 rounded up, as the CLI's --weight): g <= W x the optimum,
@@ -438,10 +439,7 @@ class PastarGPU:
         res = Result()
         rows, bufs = self._row_bufs(want_rows)
         self._ck(self.L.pg_search(self.h, C.byref(cfg), C.byref(res), rows))
-        d = res.as_dict()
-        if want_rows and res.finished:
-            d["rows"] = [b.value.decode() for b in bufs]
-        d["lower_bound"] = self.search_lower_bound()
+        d = self._result(res, bufs)
         d["weight_num"], d["weight_den"] = self.weight
         return d
 
@@ -489,10 +487,7 @@ class PastarGPU:
         res, pres, plb = Result(), (Result * k)(), (C.c_int32 * k)()
         rows, bufs = self._row_bufs(want_rows)
         self._ck(self.L.pg_search_anytime(self.h, C.byref(cfg), nums, dens, k, C.byref(res), pres, plb, rows))
-        d = res.as_dict()
-        if want_rows and res.finished:
-            d["rows"] = [b.value.decode() for b in bufs]
-        d["lower_bound"] = self.search_lower_bound()
+        d = self._result(res, bufs)
         d["phases"] = [{"weight": fr[i][0] / fr[i][1], "g": pres[i].g, "lower_bound": plb[i], "expansions": pres[i].expansions,
                         "finished": pres[i].finished} for i in range(k) if plb[i] >= 0]
         return d

@@ -4,6 +4,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <climits>
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -59,7 +61,91 @@ struct SearchCtrl {          // lives in device memory; mirrored to pinned host 
     unsigned long long phase[8]; // PG_PHASE_TIMING builds: warp-cycles per phase of the expand kernel
 };
 
-struct SearchState;
+// Owner of an instantiated CUDA graph (a captured group of search rounds).
+struct GraphExec {
+    cudaGraphExec_t exec = nullptr;
+    GraphExec() = default;
+    GraphExec(const GraphExec &) = delete;
+    GraphExec &operator=(const GraphExec &) = delete;
+    ~GraphExec() { reset(); }
+    void reset()
+    {
+        if (exec) cudaGraphExecDestroy(exec);
+        exec = nullptr;
+    }
+    explicit operator bool() const { return exec != nullptr; }
+};
+
+struct PlanEntry;
+struct SearchState {
+    int keyw = 1;            // u64 words per packed key
+    int valw = 8;            // bytes per value (4 when g, the open bit and the move mask fit 32 bits)
+    int D = 0, DL = 0;       // block dimensions, directory-line dimensions
+    int nb = 31, gs = 32;    // value layout: open bit, g shift
+    uint64_t cap = 0;        // value slots = dir_slots << D (power of two)
+    uint64_t dir_slots = 0;  // directory slots = blocks (power of two)
+    unsigned long long *d_dir = nullptr;
+    void *d_vals = nullptr;
+    unsigned long long *d_buckets = nullptr;
+    uint32_t *d_tail = nullptr;              // per bucket: entries in the chunks behind the head
+    uint32_t *d_hint = nullptr;
+    uint32_t *d_pool = nullptr;
+    unsigned long long *d_link = nullptr;    // per unit: {offset, lg} of the previous chunk of the bucket
+    uint32_t *d_free = nullptr;              // free stacks of popped chunks, one per size class
+    uint32_t free_off[16] = {0};             // first entry of class lg's stack in d_free
+    uint32_t n_units = 0;
+    PlanEntry *d_plan = nullptr;
+    uint32_t plan_cap = 0;
+    size_t bytes_dir = 0, bytes_vals = 0, bytes_pool = 0, bytes_link = 0, bytes_live = 0, bytes_surv = 0; // sizes of the cached buffers
+    SearchCtrl *d_ctrl = nullptr;
+    SearchCtrl *h_ctrl = nullptr; // pinned
+    uint32_t *d_trace = nullptr;  // backtrace output
+    unsigned long long *d_live = nullptr;  // live parents of the round: (keyw + 1) arrays of live_cap u64
+    uint64_t live_cap = 0;
+    unsigned long long *d_surv = nullptr;  // local survivors of the round: pg_xrec records
+    uint64_t surv_cap = 0;
+    unsigned long long *d_host_counts = nullptr; // record counts the host passes to insert launches
+    unsigned long long h_host_counts[64] = {0};
+    pg_search_config cfg;
+    int64_t batch_target = 0;
+    int f0 = 0, f_range = 0, ub = 0;
+    int goal_limit = 0;      // goals with g >= this are dropped (the all-advance cost + 1); weighted: every successor
+    long long inc = LLONG_MAX; // the incumbent's cost U when the search began (LLONG_MAX: none)
+    // multi-partition outboxes
+    char *d_outbox = nullptr;
+    unsigned long long *d_outbox_count = nullptr;
+    unsigned long long *h_outbox_count = nullptr;
+    uint64_t outbox_cap = 0; // records per destination
+    void *peer_inbox[16] = {nullptr};
+    unsigned long long *peer_counts[16] = {nullptr}; // P2P mode: every partition's uint64[nbuf][n_parts] "records from source s"
+    int p2p_nbuf = 1, p2p_buf = 0;                   // double-buffered inboxes: one cross-GPU barrier per round is enough
+    bool stamped = false;                            // counts carry the exchange round: receivers wait for them on the device, no barrier
+    long long xround = 0;                            // exchange rounds completed
+    bool p2p = false;
+    bool forward = false;      // P2P parent forwarding (pg_search_config.reserved == 2)
+    bool merge_expand = false; // forwarding: own and forwarded parents expanded by ONE launch after the barrier
+    size_t region_bytes = 0;   // bytes one source may write into one inbox (per buffer)
+    int xrec = 0;
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    // optional per-launch timing: event triples (before select, between, after expand), harvested at every sync
+    bool profile = false;
+    std::vector<cudaEvent_t> prof_ev;
+    size_t prof_used = 0;
+    double expand_ms = 0, select_ms = 0, claim_ms = 0, insert_ms = 0, inbox_ms = 0;
+    std::vector<cudaEvent_t> prof_ev2; // pairs around the inbox inserts
+    size_t prof_used2 = 0;
+    double kernel_ms = 0;
+    int64_t rounds = 0;
+    bool active = false;
+    bool stepwise = true;    // begun by pg_search_begin (false: by pg_search, which has finished with it)
+    // pg_run_rounds: a group of rounds captured once as a CUDA graph (every round is the same launches with the same
+    // arguments; all per-round state lives in the device control block) and replayed
+    GraphExec rounds_exec;
+    int rounds_group = 0, rounds_flimit = 0;
+    cudaStream_t rounds_stream = nullptr;
+    bool rounds_no_graph = false; // a capture failed: this search runs its rounds as plain launches
+};
+
 struct pg_ctx {
     int device = 0;
     int n = 0, npairs = 0;
@@ -115,6 +201,24 @@ int pg_launch_expand(pg_ctx *ctx, const void *d_parents, int64_t k, int vec_size
 int pg_launch_calc_h(pg_ctx *ctx, const uint16_t *d_coords, int64_t n, int32_t *d_out, cudaStream_t st);
 int pg_launch_owner(pg_ctx *ctx, const uint16_t *d_coords, int64_t n, int size, uint32_t *d_out, cudaStream_t st);
 void pg_search_free(pg_ctx *ctx);
+
+// ---- the search internals the host drivers (pg_drivers.cu) build on (pg_search.cu) ------------------------------------
+int sync_ctrl(pg_ctx *ctx); // control block to the host after a stream synchronise; a device-reported error as PG_ERR_*
+void fill_counters(const SearchState *s, pg_result *r);
+// Open / closed census of this partition's table and the min of g + h over its open entries (LLONG_MAX if none).
+int pg_census(pg_ctx *ctx, int64_t *open_size, int64_t *closed_size, long long *open_lb);
+// The parent chain from the goal to the origin: move masks origin-first, and the g stored at the goal entry.
+int pg_backtrace(pg_ctx *ctx, std::vector<uint32_t> &masks, int *goal_g);
+// Capture what `enqueue` launches on ctx->stream (thread-local mode) and instantiate it as *exec.  The captured rounds
+// have not run, so the search's round count is restored.  A capture or instantiation the driver refuses leaves *exec
+// empty and returns PG_OK; an error of `enqueue` is returned as it is.
+int pg_capture(pg_ctx *ctx, const std::function<int()> &enqueue, GraphExec *exec);
+// n rounds of a single-partition search.  allow_graph: whole groups of `group` rounds replay a CUDA graph, captured on
+// first use and again when f_limit, the stream or the group size changes; after a failed capture the search does not try
+// again.  The other rounds run as plain launches.
+int pg_run_rounds(pg_ctx *ctx, int n, int f_limit, int group, bool allow_graph);
+// g of the alignment spelled by `masks` (origin first) under the context's cost model (Node.cpp:129-152).
+long long pg_path_cost(const pg_ctx *ctx, const std::vector<uint32_t> &masks);
 
 // ---- device helpers ------------------------------------------------------------------------
 #ifdef __CUDACC__
