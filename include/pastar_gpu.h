@@ -251,6 +251,10 @@ int pg_search_status(pg_ctx *ctx, int32_t *min_open_f, int32_t *best_goal_g, pg_
 /* Closed/open table lookup for the distributed backtrace
  * (pastar_functions/PAStarDistributedBacktrace.cpp:18-214): found=0 if absent. */
 int pg_search_lookup(pg_ctx *ctx, const uint16_t *pos, int32_t *found, int32_t *g, int32_t *parenti);
+/* The same lookup for `count` coordinates (host arrays; pos is count x N): state[i] 0 absent, 1 open, 2 closed; g[i] and
+ * parenti[i] are -1 when absent.  One device thread per coordinate; no project counterpart (it serves table checks).
+ * PG_ERR_ARG, before any device work, when a position is past its sequence's length or no search is active. */
+int pg_search_lookup_batch(pg_ctx *ctx, const uint16_t *pos, int64_t count, int32_t *state, int32_t *g, int32_t *parenti);
 int pg_search_end(pg_ctx *ctx);
 /* Bounded-suboptimal (weighted) search - an opt-in extension of pg_search / pg_multi_search / pg_search_begin (the
  * reference, PAStar.cpp:626-673, only searches for the optimum).  Every later search on the context orders, prunes and

@@ -108,6 +108,7 @@ def load_library():
         "pg_search_insert_segments_dev": ([vp, vp, i64, C.POINTER(i64), i32], i32),
         "pg_search_status": ([vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(Result)], i32),
         "pg_search_lookup": ([vp, vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)], i32),
+        "pg_search_lookup_batch": ([vp, vp, i64, vp, vp, vp], i32),
         "pg_search_end": ([vp], i32),
         "pg_xrec_stride": ([vp], i32),
         "pg_search_set_weight": ([vp, C.c_int32, C.c_int32], i32),
@@ -129,8 +130,8 @@ EXPORTS = ["pg_release_cached_memory", "pg_search_note_rounds", "pg_search_set_d
            "pg_ctx_set_stream", "pg_search_rounds", "pg_search_profile", "pg_abi_version", "pg_last_error", "pg_default_cost_table", "pg_host_weights", "pg_ctx_create", "pg_ctx_destroy",
            "pg_build_pair_tables", "pg_pair_table_shape", "pg_copy_pair_table", "pg_calculate_h", "pg_configure_hash",
            "pg_owner", "pg_expand_batch", "pg_expand_batch_dev", "pg_search", "pg_search_begin", "pg_search_round",
-           "pg_search_outbox", "pg_search_insert_dev", "pg_search_status", "pg_search_lookup", "pg_search_end",
-           "pg_xrec_stride", "pg_search_set_weight", "pg_search_lower_bound", "pg_score_alignment", "pg_search_set_incumbent",
+           "pg_search_outbox", "pg_search_insert_dev", "pg_search_status", "pg_search_lookup", "pg_search_lookup_batch",
+           "pg_search_end", "pg_xrec_stride", "pg_search_set_weight", "pg_search_lower_bound", "pg_score_alignment", "pg_search_set_incumbent",
            "pg_search_anytime"]
 
 WEIGHT_DEN = 1024
@@ -576,6 +577,15 @@ class PastarGPU:
         f, g, p = C.c_int32(), C.c_int32(), C.c_int32()
         self._ck(self.L.pg_search_lookup(self.h, a.ctypes.data, C.byref(f), C.byref(g), C.byref(p)))
         return (g.value, p.value) if f.value else None
+
+    def search_lookup_many(self, pos):
+        """pg_search_lookup_batch: (state, g, parenti) int32 arrays for K coordinates (K x N); state 0 absent, 1 open,
+        2 closed; g and parenti -1 where absent."""
+        a = np.ascontiguousarray(pos, dtype=np.uint16).reshape(-1, self.n)
+        k = a.shape[0]
+        state, g, par = (np.zeros(k, dtype=np.int32) for _ in range(3))
+        self._ck(self.L.pg_search_lookup_batch(self.h, a.ctypes.data, k, state.ctypes.data, g.ctypes.data, par.ctypes.data))
+        return state, g, par
 
     def search_end(self):
         self._ck(self.L.pg_search_end(self.h))

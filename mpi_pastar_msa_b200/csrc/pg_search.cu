@@ -1796,6 +1796,31 @@ __global__ void lookup_kernel(const __grid_constant__ DevProblem p, const __grid
     out[3] = val_closed<VALW>(d, val) ? 0 : 1;
 }
 
+// The same lookup for many coordinates, one thread each: state 0 absent / 1 open / 2 closed, g and move mask (-1 when
+// absent).  Read-only, so it may run between rounds; table checks look up whole lattices or frontiers through it.
+template <int KEYW, int VALW>
+__global__ void lookup_batch_kernel(const __grid_constant__ DevProblem p, const __grid_constant__ DevSearch d, const uint16_t *pos,
+                                    long long count, int *state, int *g, int *parenti)
+{
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < count; i += (long long)gridDim.x * blockDim.x) {
+        Key<KEYW> key = Key<KEYW>::zero();
+        for (int k = 0; k < p.n; k++) key.add_val((unsigned)pos[i * p.n + k], k * p.key_bits);
+        int st = 0, gv = -1, pm = -1;
+        const unsigned long long slot = table_find<KEYW>(d, key, false);
+        if (slot != ~0ull) {
+            const typename ValT<VALW>::T val = *val_ptr<VALW>(d, slot);
+            if (val != 0) {
+                st = val_closed<VALW>(d, val) ? 2 : 1;
+                gv = (int)val_g<VALW>(d, val);
+                pm = (int)val_mask<VALW>(d, val);
+            }
+        }
+        state[i] = st;
+        g[i] = gv;
+        parenti[i] = pm;
+    }
+}
+
 // Count open / closed entries at the end (PAStar.cpp:591-619 report): every value of every block in use.  out[0] / out[1]
 // count open / closed entries; out[2] (set to LLONG_MAX by the caller) receives the min of g + h (unweighted h) over the open
 // entries, the open-list part of the search's lower bound: the coordinate is decoded from the block's directory key and
@@ -2739,6 +2764,44 @@ extern "C" int pg_search_lookup(pg_ctx *ctx, const uint16_t *pos, int32_t *found
     if (g) *g = h[1];
     if (parenti) *parenti = h[2];
     return PG_OK;
+}
+
+extern "C" int pg_search_lookup_batch(pg_ctx *ctx, const uint16_t *pos, int64_t count, int32_t *state, int32_t *g, int32_t *parenti)
+{
+    if (!ctx || !ctx->search || count < 0 || (count > 0 && (!pos || !state || !g || !parenti))) return PG_ERR_ARG;
+    const int n = ctx->n;
+    for (int64_t i = 0; i < count; i++)
+        for (int k = 0; k < n; k++)
+            if ((int)pos[i * n + k] > ctx->len[k])
+                return pg_fail(ctx, PG_ERR_ARG, "pg_search_lookup_batch: coordinate " + std::to_string(i) + " has position " +
+                                                    std::to_string(pos[i * n + k]) + " in sequence " + std::to_string(k) +
+                                                    ", past its length " + std::to_string(ctx->len[k]));
+    if (count == 0) return PG_OK;
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
+    SearchState *s = ctx->search;
+    const int64_t chunk = std::min<int64_t>(count, 1 << 22); // bounded scratch: 4 Mi coordinates per launch
+    void *buf = nullptr;
+    PG_CUDA(ctx, cudaMalloc(&buf, (size_t)chunk * (2 * n + 12)));
+    int *d_out = (int *)buf;
+    uint16_t *d_pos = (uint16_t *)(d_out + 3 * chunk);
+    int rc = PG_OK;
+    for (int64_t b = 0; b < count && rc == PG_OK; b += chunk) {
+        const int64_t k = std::min(chunk, count - b);
+        cudaError_t e = cudaMemcpyAsync(d_pos, pos + b * n, (size_t)k * n * 2, cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess) {
+            const unsigned grid = (unsigned)std::min<int64_t>((k + 255) / 256, (int64_t)ctx->sm_count * 16);
+            PG_DISPATCH_KV(s, (lookup_batch_kernel<KW, VW><<<grid, 256, 0, ctx->stream>>>(ctx->dp, dev_search(ctx), d_pos, (long long)k,
+                                                                                          d_out, d_out + chunk, d_out + 2 * chunk)));
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess) e = cudaMemcpyAsync(state + b, d_out, (size_t)k * 4, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(g + b, d_out + chunk, (size_t)k * 4, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(parenti + b, d_out + 2 * chunk, (size_t)k * 4, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) rc = pg_fail(ctx, PG_ERR_CUDA, std::string("pg_search_lookup_batch: ") + cudaGetErrorString(e));
+    }
+    cudaFree(buf);
+    return rc;
 }
 
 extern "C" int pg_search_end(pg_ctx *ctx)

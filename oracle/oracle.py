@@ -59,6 +59,9 @@ def lib():
         L.po_get_neigh.restype = C.c_int
         L.po_astar.argtypes = [C.c_void_p, C.c_int64, C.POINTER(SearchResult), C.POINTER(C.c_char_p)]
         L.po_astar.restype = C.c_int
+        L.po_astar_settled.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.POINTER(C.c_int32), C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.POINTER(SearchResult)]
+        L.po_astar_settled.restype = C.c_int64
         _lib = L
     return _lib
 
@@ -165,6 +168,22 @@ class Problem:
         if want_rows and res.finished:
             d["rows"] = [b.value.decode() for b in bufs]
         return d
+
+    def astar_settled(self, budget=0, cap=None):
+        """The serial A* of astar() for `budget` pops (0: to the goal), then its settled set: (F, pos, g, parenti), where
+        F is the f of the best live open entry and pos[k] / g[k] / parenti[k] are the closed nodes with f < F."""
+        if cap is None:
+            cap = budget + 1 if budget > 0 else 1 << 16
+        while True:
+            pos = np.zeros((cap, self.n), dtype=np.uint16)
+            g = np.zeros(cap, dtype=np.int32)
+            par = np.zeros(cap, dtype=np.int32)
+            F, res = C.c_int32(), SearchResult()
+            k = lib().po_astar_settled(self.h, budget, cap, C.byref(F), pos.ctypes.data, g.ctypes.data, par.ctypes.data,
+                                       C.byref(res))
+            if k <= cap:
+                return F.value, pos[:k], g[:k], par[:k]
+            cap = k
 
 
 def owner(pos, hash_type="FZORDER", shift=12, size=1):

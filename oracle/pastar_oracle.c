@@ -742,7 +742,9 @@ static void open_conditional_enqueue(astar *a, const uint16_t *pos, int32_t g, i
     heap_push(a, h);
 }
 
-int po_astar(const po_problem *p, int64_t budget, po_search_result *res, char **rows)
+/* The search loop of po_astar: runs until the goal is popped, the open list empties or `budget` pops, and leaves the
+ * table and heap in *a for the caller to read and free. */
+static void astar_run(const po_problem *p, int64_t budget, po_search_result *res, astar *out)
 {
     int n = p->n;
     astar a;
@@ -797,6 +799,17 @@ int po_astar(const po_problem *p, int64_t budget, po_search_result *res, char **
         if (budget > 0 && res->pops >= budget) break;
     }
     res->open_size = open_live;
+    free(succ);
+    *out = a;
+}
+
+int po_astar(const po_problem *p, int64_t budget, po_search_result *res, char **rows)
+{
+    int n = p->n;
+    uint16_t fin[PO_MAX_SEQ] = {0};
+    for (int i = 0; i < n; i++) fin[i] = (uint16_t)p->len[i];
+    astar a;
+    astar_run(p, budget, res, &a);
     if (res->finished && rows) {
         /* backtrace.cpp:44-69 */
         int total = 0;
@@ -824,8 +837,35 @@ int po_astar(const po_problem *p, int64_t budget, po_search_result *res, char **
         }
         free(buf);
     }
-    free(succ);
     free(a.tab);
     free(a.heap);
     return 0;
+}
+
+int64_t po_astar_settled(const po_problem *p, int64_t budget, int64_t cap, int32_t *F_out, uint16_t *pos, int32_t *g,
+                         int32_t *parenti, po_search_result *res)
+{
+    int n = p->n;
+    astar a;
+    astar_run(p, budget, res, &a);
+    int32_t F = INT32_MAX;
+    for (uint64_t i = 0; i < a.hn; i++) { /* the best live entry: skip superseded ones */
+        const anode *e = &a.tab[a.heap[i].slot];
+        if (e->state == 1 && e->stamp == a.heap[i].stamp && a.heap[i].f < F) F = a.heap[i].f;
+    }
+    *F_out = F;
+    int64_t k = 0;
+    for (uint64_t i = 0; i < a.cap; i++) {
+        const anode *e = &a.tab[i];
+        if (e->state != 2 || e->f >= F) continue;
+        if (k < cap) {
+            memcpy(pos + (size_t)k * n, e->pos, sizeof(uint16_t) * n);
+            g[k] = e->g;
+            parenti[k] = e->parenti;
+        }
+        k++;
+    }
+    free(a.tab);
+    free(a.heap);
+    return k;
 }

@@ -70,6 +70,13 @@ int po_get_neigh(const po_problem *p, const uint16_t *pos, int32_t g, int32_t pa
  * that many pops.  rows (n strings of at least sum(lens)+1 bytes) may be NULL. */
 int po_astar(const po_problem *p, int64_t budget, po_search_result *res, char **rows);
 
+/* The settled set of the same search after `budget` pops (0: run to the goal).  *F_out receives the f of the best live
+ * open entry (INT32_MAX when the open list is empty); every closed node with f < *F_out is written as pos[k * n ..],
+ * g[k], parenti[k], the first `cap` of them.  Returns how many there are (more than cap: call again with more room).
+ * Under a consistent heuristic these are exactly the nodes with g* + h < F, each with g == g*. */
+int64_t po_astar_settled(const po_problem *p, int64_t budget, int64_t cap, int32_t *F_out, uint16_t *pos, int32_t *g,
+                         int32_t *parenti, po_search_result *res);
+
 #ifdef __cplusplus
 }
 #endif
