@@ -301,6 +301,30 @@ int pg_search_set_incumbent(pg_ctx *ctx, const char *const *rows, int32_t cols);
  * what it was before the call and the incumbent is the alignment returned. */
 int pg_search_anytime(pg_ctx *ctx, const pg_search_config *cfg, const int32_t *weight_num, const int32_t *weight_den, int n_phases,
                       pg_result *res, pg_result *phase_res, int32_t *phase_lb, char *const *rows);
+/* Layered search (breadth-first heuristic search with divide-and-conquer reconstruction, Zhou & Hansen 2006; no reference
+ * counterpart).  The lattice is swept level by level (level = sum of the coordinates): each node is expanded once with
+ * its final g, only the N + 1 levels in flight are held, and successors with g + h >= U are pruned.  Top-level passes
+ * raise U (BFIDA*) until one reaches the goal with g < U: that g is the optimum.  The alignment is then rebuilt by
+ * narrower passes between relay nodes.  Exact search with gap_open == gap_ext only.
+ *   cfg->table_capacity: coordinates the N + 1 level tables of a pass hold at once (each level at most 1 / (N + 1) of it;
+ *                        0 = 2^22); a level that does not fit gives PG_ERR_CAPACITY.  cfg->max_expansions (0: none): a
+ *                        budget over every pass.  The other fields are ignored.
+ *   res: finished 1 (optimal; g = f = C*), 2 (an incumbent is set and nothing is cheaper: it is returned and the lower
+ *        bound is U), 0 (the budget ran out: the lower bound is the best failed pass's f_min or h(start); when it runs
+ *        out while the alignment is being rebuilt, C* is proved and the lower bound is C*, but g = -1 and no rows).
+ *        expansions / generated / inserted are summed over all passes, rounds = levels swept.
+ *   rows (may be NULL): as pg_search.  NULL also skips the reconstruction: the cost alone, align_len = 0.
+ *   stats (may be NULL): see pg_layered_stats.
+ * Honours pg_search_set_incumbent (its cost caps U).  PG_ERR_UNSUPPORTED for gap_open != gap_ext or a key over 127 bits,
+ * PG_ERR_ARG for a search weight other than 1, PG_ERR_STATE without pair tables or while a step-wise search is active.
+ * Afterwards pg_search_lower_bound gives the certified bound. */
+typedef struct {
+    int32_t iterations, first_bound, last_bound, depth; /* top-level passes, their first / last U, deepest recursion   */
+    int64_t passes, levels;             /* all passes incl. reconstruction; levels swept over all of them              */
+    int64_t max_level_nodes, max_held;  /* most coordinates in one level / in all level tables at once                */
+    int64_t peak_bytes, top_expansions; /* device bytes the mode allocated; expansions of the last top-level pass      */
+} pg_layered_stats;
+int pg_search_layered(pg_ctx *ctx, const pg_search_config *cfg, pg_result *res, pg_layered_stats *stats, char *const *rows);
 /* bytes per exchanged successor record for this context */
 int pg_xrec_stride(const pg_ctx *ctx);
 

@@ -11,6 +11,7 @@ Reference interface                                   -> here
   PAStar::pa_star (PAStar.cpp:626-673)                 -> .search
   (no reference counterpart: bounded-suboptimal search) -> .search(weight=W) / .search_set_weight / .search_lower_bound
   (no reference counterpart: incumbent / anytime search) -> .score_alignment / .search(incumbent=rows) / .anytime_search
+  (no reference counterpart: layered search)           -> .layered_search
 """
 import ctypes as C
 import math
@@ -43,6 +44,15 @@ class Result(C.Structure):
                 ("inserted", C.c_int64), ("seconds", C.c_double), ("kernel_ms", C.c_double), ("expand_ms", C.c_double),
                 ("select_ms", C.c_double), ("claim_ms", C.c_double), ("insert_ms", C.c_double),
                 ("survivors", C.c_int64), ("inbox_ms", C.c_double)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class LayeredStats(C.Structure):
+    _fields_ = [("iterations", C.c_int32), ("first_bound", C.c_int32), ("last_bound", C.c_int32), ("depth", C.c_int32),
+                ("passes", C.c_int64), ("levels", C.c_int64), ("max_level_nodes", C.c_int64), ("max_held", C.c_int64),
+                ("peak_bytes", C.c_int64), ("top_expansions", C.c_int64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -117,6 +127,7 @@ def load_library():
         "pg_search_set_incumbent": ([vp, C.POINTER(C.c_char_p), C.c_int32], i32),
         "pg_search_anytime": ([vp, C.POINTER(SearchConfig), C.POINTER(C.c_int32), C.POINTER(C.c_int32), i32, C.POINTER(Result),
                                C.POINTER(Result), C.POINTER(C.c_int32), C.POINTER(C.c_char_p)], i32),
+        "pg_search_layered": ([vp, C.POINTER(SearchConfig), C.POINTER(Result), C.POINTER(LayeredStats), C.POINTER(C.c_char_p)], i32),
     }
     for name, (args, res) in sig.items():
         f = getattr(L, name)
@@ -132,7 +143,7 @@ EXPORTS = ["pg_release_cached_memory", "pg_search_note_rounds", "pg_search_set_d
            "pg_owner", "pg_expand_batch", "pg_expand_batch_dev", "pg_search", "pg_search_begin", "pg_search_round",
            "pg_search_outbox", "pg_search_insert_dev", "pg_search_status", "pg_search_lookup", "pg_search_lookup_batch",
            "pg_search_end", "pg_xrec_stride", "pg_search_set_weight", "pg_search_lower_bound", "pg_score_alignment", "pg_search_set_incumbent",
-           "pg_search_anytime"]
+           "pg_search_anytime", "pg_search_layered"]
 
 WEIGHT_DEN = 1024
 
@@ -491,6 +502,24 @@ class PastarGPU:
         d = self._result(res, bufs)
         d["phases"] = [{"weight": fr[i][0] / fr[i][1], "g": pres[i].g, "lower_bound": plb[i], "expansions": pres[i].expansions,
                         "finished": pres[i].finished} for i in range(k) if plb[i] >= 0]
+        return d
+
+    def layered_search(self, incumbent=None, table_capacity=0, max_expansions=0, want_rows=True):
+        """pg_search_layered: exact search level by level under a raised bound, holding N + 1 lattice levels instead of
+        every coordinate generated.  table_capacity: coordinates the level tables hold at once (0: 2^22); max_expansions:
+        a budget over all passes.  incumbent (alignment rows): set first (search_set_incumbent), as search().
+        want_rows=False returns the cost alone (the alignment is not rebuilt).  Returns search()'s dict with lower_bound
+        and `layered`, the pass statistics (pg_layered_stats)."""
+        if incumbent is not None:
+            self.search_set_incumbent(incumbent)
+        cfg = SearchConfig(1, 0, table_capacity, 0, max_expansions, 0, 0)
+        res, st = Result(), LayeredStats()
+        rows, bufs = self._row_bufs(want_rows)
+        self._ck(self.L.pg_search_layered(self.h, C.byref(cfg), C.byref(res), C.byref(st), rows))
+        d = self._result(res, bufs)
+        if res.finished == 1 and not want_rows:
+            d.pop("rows", None)
+        d["layered"] = st.as_dict()
         return d
 
     def search_lower_bound(self):

@@ -21,7 +21,7 @@ BIN = os.path.join(HERE, "bin", "pastar")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 CXX = os.environ.get("CXX", "g++")
 
-CU_SOURCES = ["pg_api.cu", "pg_pairdp.cu", "pg_expand.cu", "pg_primer.cu", "pg_search.cu", "pg_drivers.cu"]
+CU_SOURCES = ["pg_api.cu", "pg_pairdp.cu", "pg_expand.cu", "pg_primer.cu", "pg_search.cu", "pg_drivers.cu", "pg_layered.cu"]
 HOST_SOURCES = ["host/pg_host_weights.cpp"]
 CLI_SOURCES = ["host/pastar_main.cpp"]
 NVCC_FLAGS = (["-DPG_PHASE_TIMING"] if PHASE else []) + os.environ.get("PG_EXTRA_NVCC", "").split() + ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--expt-relaxed-constexpr",

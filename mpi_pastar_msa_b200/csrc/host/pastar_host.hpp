@@ -411,6 +411,7 @@ struct PAStarOpt { // PAStar.h:87-112, plus the GPU-side knobs (new, do not chan
     std::string incumbent;                  // --incumbent FILE: aligned FASTA of a known alignment (upper bound of the search)
     std::vector<std::string> incumbent_rows; // its rows, checked against the input before any device call
     std::vector<int32_t> anytime_num;        // --anytime W1,W2,...: one weighted phase per weight, num / 1024 (empty: not given)
+    bool layered = false;                    // --layered: pg_search_layered instead of pg_search (one GPU, exact)
 };
 
 int read_fasta_file(const std::string &name);
@@ -449,7 +450,9 @@ class PAStar {
         for (int i = 0; i < N; i++) rowp[i] = bufs[i].data();
         const int wden = 1024;
         int32_t lower_bound = 0;
-        const bool bounded = options.weight_num || !options.incumbent_rows.empty() || !options.anytime_num.empty();
+        const bool bounded = options.weight_num || !options.incumbent_rows.empty() || !options.anytime_num.empty() || options.layered;
+        pg_layered_stats lst;
+        memset(&lst, 0, sizeof(lst));
         std::vector<const char *> inc(N);
         for (int i = 0; i < (int)options.incumbent_rows.size(); i++) inc[i] = options.incumbent_rows[i].c_str();
         const int inc_cols = options.incumbent_rows.empty() ? 0 : (int)options.incumbent_rows[0].size();
@@ -467,6 +470,8 @@ class PAStar {
                 h->check(pg_search_anytime(h->ctx, &cfg, options.anytime_num.data(), dens.data(), n_phases, &res, phase_res.data(),
                                            phase_lb.data(), rowp.data()),
                          "pg_search_anytime");
+            } else if (options.layered) {
+                h->check(pg_search_layered(h->ctx, &cfg, &res, &lst, rowp.data()), "pg_search_layered");
             } else {
                 h->check(pg_search(h->ctx, &cfg, &res, rowp.data()), "pg_search");
             }
@@ -487,7 +492,7 @@ class PAStar {
         // weighted, incumbent-bounded and anytime search: the optimum is at least the lower bound, so g / bound is the
         // certified ratio to it (1: the alignment is proved optimal)
         auto print_bound = [&]() {
-            if (!(options.weight_num > wden || inc_cols || n_phases)) return;
+            if (!(options.weight_num > wden || inc_cols || n_phases || options.layered)) return;
             std::cout << "Lower bound: " << lower_bound;
             if (res.finished) std::cout << "\tg / lower bound: " << std::fixed << std::setprecision(4) << (double)res.g / lower_bound;
             std::cout << std::endl;
@@ -496,6 +501,11 @@ class PAStar {
                     std::cout << "Anytime phase " << k + 1 << ": weight " << std::defaultfloat << std::setprecision(6) << (double)options.anytime_num[k] / wden
                               << ", score " << phase_res[k].g << ", lower bound " << phase_lb[k] << ", expansions " << phase_res[k].expansions
                               << std::endl;
+            if (options.layered)
+                std::cout << "Layered: " << lst.iterations << " top-level passes (bound " << lst.first_bound << " .. " << lst.last_bound
+                          << "), " << lst.passes << " passes, " << lst.levels << " levels, depth " << lst.depth << ", widest level "
+                          << lst.max_level_nodes << ", at most " << lst.max_held << " coordinates held, " << lst.peak_bytes
+                          << " bytes" << std::endl;
         };
         if (!res.finished) {
             std::cout << "Search stopped at the expansion budget: " << res.expansions << " expansions, no alignment.\n";
@@ -551,6 +561,11 @@ class PAStar {
                 }
                 js << "]";
             }
+            if (options.layered)
+                js << ", \"layered\": {\"iterations\": " << lst.iterations << ", \"first_bound\": " << lst.first_bound
+                   << ", \"last_bound\": " << lst.last_bound << ", \"depth\": " << lst.depth << ", \"passes\": " << lst.passes
+                   << ", \"levels\": " << lst.levels << ", \"max_level_nodes\": " << lst.max_level_nodes << ", \"max_held\": "
+                   << lst.max_held << ", \"peak_bytes\": " << lst.peak_bytes << ", \"top_expansions\": " << lst.top_expansions << "}";
             js << ", \"total\": ";
             one(res);
             js << ", \"partitions\": [";

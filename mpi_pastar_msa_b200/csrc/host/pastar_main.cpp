@@ -2,7 +2,7 @@
 //
 //   pastar [-t N] [-s SHIFT] [-y FZORDER|FSUM|PZORDER|PSUM] [-v] [-h] [--memory_debug] file.fasta
 //   new, optional: [-g/--gpus N] [--batch K] [--table_capacity SLOTS] [--max_expansions E] [--metrics_json FILE] [--weight W]
-//                  [--incumbent FILE] [--anytime W1,W2,...]
+//                  [--incumbent FILE] [--anytime W1,W2,...] [--layered]
 //
 // Same flags, exit codes (0 ok, 1 usage / not a regular file, -1 on exception) and stdout format as the reference
 // (phase timers, "Final Score:", "Similarity:", wrapped alignment, "Total nodes count:" table).  No MPI: the
@@ -70,6 +70,8 @@ static void usage(const char *argv0)
               << "                                prove it optimal\n"
               << "  --anytime arg                 comma-separated weights (1..16), one search per weight, each bounded\n"
               << "                                by the best alignment so far (one GPU)\n"
+              << "  --layered                     exact search level by level: holds a few lattice levels, not every\n"
+              << "                                coordinate generated (one GPU; composes with --incumbent)\n"
               << std::endl;
 }
 
@@ -92,7 +94,7 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
     // Boost.ProgramOptions' default style lets a long option be shortened to any unambiguous prefix ("--thr 4", "--hash_t=FSUM")
     static const char *const long_names[] = {"version", "help", "memory_debug", "threads", "hash_shift", "hash_type", "gpus",
                                              "batch", "table_capacity", "max_expansions", "metrics_json", "weight",
-                                             "incumbent", "anytime"};
+                                             "incumbent", "anytime", "layered"};
     auto canonical = [&](const std::string &arg) -> std::string {
         if (arg.size() < 3 || arg.compare(0, 2, "--") != 0) return arg;
         const size_t eq = arg.find('=');
@@ -136,6 +138,7 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
         else if (is_long(a, "metrics_json")) opt.metrics_json = value(i, a, "metrics_json");
         else if (is_long(a, "weight")) opt.weight_num = weight_num(value(i, a, "weight"), "weight");
         else if (is_long(a, "incumbent")) opt.incumbent = value(i, a, "incumbent");
+        else if (a == "--layered") opt.layered = true;
         else if (is_long(a, "anytime")) {
             const std::string v = value(i, a, "anytime");
             opt.anytime_num.clear();
@@ -160,6 +163,10 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
     else throw std::invalid_argument("the argument for option '--hash_type' is invalid");
     if (!opt.anytime_num.empty() && opt.weight_num) throw std::invalid_argument("option '--anytime' cannot be combined with '--weight'");
     if (!opt.anytime_num.empty() && opt.gpus != 1) throw std::invalid_argument("option '--anytime' runs on one GPU (--gpus 1)");
+    if (opt.layered && !opt.anytime_num.empty()) throw std::invalid_argument("option '--layered' cannot be combined with '--anytime'");
+    if (opt.layered && opt.weight_num && opt.weight_num != 1024)
+        throw std::invalid_argument("option '--layered' cannot be combined with '--weight' other than 1");
+    if (opt.layered && opt.gpus != 1) throw std::invalid_argument("option '--layered' cannot be combined with '--gpus' above 1");
     if (version) {
         std::cout << "msa_pastar, version 1.0\n";
         std::exit(0);

@@ -7,6 +7,7 @@
 #include <atomic>
 #include <chrono>
 #include <climits>
+#include <cmath>
 #include <cstring>
 #include <thread>
 #include <vector>
@@ -230,6 +231,275 @@ extern "C" int pg_search(pg_ctx *ctx, const pg_search_config *cfg_in, pg_result 
     ctx->lb_valid = true;
     res->seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     return PG_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// pg_search_layered: breadth-first heuristic search (Zhou & Hansen, AIJ 2006) with an iteratively raised bound (BFIDA*)
+// and divide-and-conquer reconstruction over relay nodes.  The level passes are in pg_layered.cu; DESIGN.md §4.4c.
+// ---------------------------------------------------------------------------------------------------------------------
+namespace {
+
+// c(pos, mask) under the context's cost model with gap_open == gap_ext (the incoming move does not matter)
+long long move_cost(const pg_ctx *ctx, const int *pos, uint32_t m)
+{
+    const DevProblem &p = ctx->dp;
+    long long sum = 0;
+    for (int pr = 0; pr < p.npairs; pr++) {
+        const int x = p.pa[pr], y = p.pb[pr];
+        const int mx = (m >> x) & 1, my = (m >> y) & 1;
+        const int c = mx && my ? ctx->cost[(unsigned char)ctx->seqs[x][pos[x]] * 90 + (unsigned char)ctx->seqs[y][pos[y]]]
+                               : (mx || my ? p.gap_ext : p.gap_gap);
+        sum += (long long)c * p.w[pr];
+    }
+    return sum;
+}
+
+// Bin width of a top-level pass at bound U: the bins below the last one span 2 (U - h(start)), so the bound can at most
+// triple its distance from h(start) in one step.
+int bin_width(long long U, long long h0)
+{
+    return (int)std::max(1LL, (2 * std::max(1LL, U - h0) + PG_LAYERED_BINS - 2) / (PG_LAYERED_BINS - 1));
+}
+
+// The next bound of the top-level passes: the least bin edge U + (b + 1) w below which the failed pass pruned at least
+// sqrt(expansions x generated) records, else the top of the bins, or f_min + 1 when every pruned record lies above them;
+// at most `cap`.  Always above the pass's f_min.  (On kinase a target of `expansions` records grew the passes by about
+// 10 % each, 89 passes; a target of `generated` overshot C* by 2.4 % and expanded ten times the nodes below it.)
+long long next_bound(const LayPassOut &o, int U, int w, long long cap)
+{
+    unsigned long long cum = 0;
+    const int nb = (int)o.hist.size();
+    const unsigned long long target = std::max<unsigned long long>(1, (unsigned long long)std::sqrt((double)o.expansions * (double)o.generated));
+    for (int b = 0; b + 1 < nb; b++) {
+        cum += o.hist[b];
+        if (cum >= target) return std::min(cap, (long long)U + (long long)(b + 1) * w);
+    }
+    return std::min(cap, std::max((long long)U + (long long)(nb - 1) * w, (long long)o.fmin + 1));
+}
+
+struct Layered {
+    pg_ctx *ctx;
+    LayeredState *L = nullptr;
+    int retain_levels = 0;
+    int C = 0;                 // the optimum, bound of every reconstruction pass
+    int64_t budget = 0, used = 0;
+    bool out_of_budget = false;
+    pg_result *res;
+    pg_layered_stats st;
+
+    int pass(const LayPassIn &in, LayPassOut &o)
+    {
+        if (budget > 0 && used >= budget) {
+            o = LayPassOut();
+            out_of_budget = true;
+            return PG_OK;
+        }
+        const int rc = pg_layered_pass(ctx, L, in, budget > 0 ? budget - used : 0, o);
+        if (rc != PG_OK) return rc;
+        used += o.expansions;
+        res->expansions += o.expansions;
+        res->generated += o.generated;
+        res->inserted += o.inserted;
+        st.passes++;
+        st.levels += o.levels;
+        st.max_level_nodes = std::max(st.max_level_nodes, o.max_level_nodes);
+        st.max_held = std::max(st.max_held, o.max_held);
+        if (o.aborted || (budget > 0 && used >= budget && !o.reached)) out_of_budget = true;
+        return PG_OK;
+    }
+
+    // append the moves of an optimal path from s (g*(s) = gs) to t (g*(t) = gt), both on an optimal alignment
+    int solve(const int *s, const int *t, int gs, int gt, int depth, std::vector<uint32_t> &masks)
+    {
+        int ls = 0, lt = 0;
+        for (int i = 0; i < ctx->n; i++) {
+            ls += s[i];
+            lt += t[i];
+        }
+        if (ls == lt) return PG_OK;
+        st.depth = std::max(st.depth, depth);
+        LayPassIn in;
+        memcpy(in.s, s, sizeof(in.s));
+        memcpy(in.t, t, sizeof(in.t));
+        in.g0 = gs;
+        in.U = C;
+        in.hist_w = 1;
+        in.strict = false;
+        in.retain = lt - ls + 1 <= retain_levels;
+        in.mid = (ls + lt) / 2;
+        LayPassOut o;
+        int rc = pass(in, o);
+        if (rc != PG_OK || out_of_budget) return rc;
+        if (!o.reached || o.goal_g != gt)
+            return pg_fail(ctx, PG_ERR_STATE, "pg_search_layered: a reconstruction pass missed the optimal g of its corner");
+        if (in.retain) {
+            std::vector<uint32_t> m;
+            if ((rc = pg_layered_trace(ctx, L, in, m)) != PG_OK) return rc;
+            masks.insert(masks.end(), m.begin(), m.end());
+            return PG_OK;
+        }
+        return split(s, t, gs, gt, o, depth, masks);
+    }
+
+    // s .. p, the crossing move p -> x, x .. t, with x = o's relay
+    int split(const int *s, const int *t, int gs, int gt, const LayPassOut &o, int depth, std::vector<uint32_t> &masks)
+    {
+        int p[PG_MAX_SEQ] = {0};
+        for (int i = 0; i < ctx->n; i++) p[i] = o.relay[i] - ((o.relay_mask >> i) & 1);
+        const int gp = (int)(o.relay_g - move_cost(ctx, p, o.relay_mask));
+        int rc = solve(s, p, gs, gp, depth + 1, masks);
+        if (rc != PG_OK || out_of_budget) return rc;
+        masks.push_back(o.relay_mask);
+        return solve(o.relay, t, o.relay_g, gt, depth + 1, masks);
+    }
+};
+
+} // namespace
+
+extern "C" int pg_search_layered(pg_ctx *ctx, const pg_search_config *cfg_in, pg_result *res, pg_layered_stats *stats, char *const *rows)
+{
+    if (!ctx || !res) return PG_ERR_ARG;
+    int rc = refuse_while_stepwise(ctx, "pg_search_layered");
+    if (rc != PG_OK) return rc;
+    if (!ctx->tables_built) return pg_fail(ctx, PG_ERR_STATE, "pg_search_layered: pg_build_pair_tables has not run");
+    if (ctx->dp.gap_open != ctx->dp.gap_ext)
+        return pg_fail(ctx, PG_ERR_UNSUPPORTED, "pg_search_layered: gap_open != gap_ext (a coordinate is then not a state)");
+    if (ctx->wnum != 1 || ctx->wsh != 0) return pg_fail(ctx, PG_ERR_ARG, "pg_search_layered: exact search only (search weight 1)");
+    if (ctx->n * ctx->dp.key_bits > 127) return pg_fail(ctx, PG_ERR_UNSUPPORTED, "packed coordinate key exceeds 127 bits");
+    const pg_search_config cfg = config_or_zero(cfg_in);
+    if (cfg.table_capacity < 0 || cfg.max_expansions < 0) return pg_fail(ctx, PG_ERR_ARG, "pg_search_layered: negative capacity or budget");
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
+    memset(res, 0, sizeof(*res));
+    res->g = res->f = -1;
+    ctx->lb_valid = false;
+    const auto t0 = std::chrono::steady_clock::now();
+    const int n = ctx->n;
+    int origin[PG_MAX_SEQ] = {0}, goal[PG_MAX_SEQ] = {0}, D = 0;
+    for (int i = 0; i < n; i++) {
+        goal[i] = ctx->len[i];
+        D += ctx->len[i];
+    }
+    std::vector<uint16_t> zero(n, 0);
+    int32_t h0 = 0;
+    if ((rc = pg_calculate_h(ctx, zero.data(), 1, &h0)) != PG_OK) return rc;
+    std::vector<uint32_t> all_advance; // the search's UB, as pg_search_begin
+    for (int c = 0, mx = *std::max_element(ctx->len, ctx->len + n); c < mx; c++) {
+        uint32_t m = 0;
+        for (int i = 0; i < n; i++) m |= (uint32_t)(c < ctx->len[i]) << i;
+        all_advance.push_back(m);
+    }
+    const long long ub = pg_path_cost(ctx, all_advance);
+    const bool has_inc = ctx->inc_cost >= 0;
+    const long long cap = has_inc ? ctx->inc_cost : ub + 1; // strict bounds: the last pass keeps g + h < cap
+    if (cap > INT_MAX - 1) return pg_fail(ctx, PG_ERR_UNSUPPORTED, "pg_search_layered: the upper bound does not fit 31 bits");
+
+    // PG_LAYERED_DEEP: recurse down to single moves; PG_LAYERED_RETAIN: reconstruct in one retain pass over the lattice
+    const bool deep = getenv("PG_LAYERED_DEEP") != nullptr, retain_all = getenv("PG_LAYERED_RETAIN") != nullptr;
+    Layered S;
+    S.ctx = ctx;
+    S.res = res;
+    memset(&S.st, 0, sizeof(S.st));
+    S.retain_levels = retain_all ? D + 1 : (deep ? 1 : 4 * (n + 1));
+    S.budget = cfg.max_expansions;
+    const int64_t capacity = cfg.table_capacity > 0 ? cfg.table_capacity : (1LL << 22);
+    if ((rc = pg_layered_open(ctx, std::max<int64_t>(1, capacity / (n + 1)), S.retain_levels, &S.L)) != PG_OK) {
+        pg_layered_close(ctx, S.L);
+        return rc;
+    }
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    auto finish = [&](int code) {
+        if (ev0) cudaEventDestroy(ev0);
+        if (ev1) cudaEventDestroy(ev1);
+        pg_layered_close(ctx, S.L);
+        return code;
+    };
+#define LAY_CHECK(expr)                 \
+    do {                                \
+        if ((rc = (expr)) != PG_OK)     \
+            return finish(rc);          \
+    } while (0)
+    if (cudaEventCreate(&ev0) != cudaSuccess || cudaEventCreate(&ev1) != cudaSuccess || cudaEventRecord(ev0, ctx->stream) != cudaSuccess)
+        return finish(pg_fail(ctx, PG_ERR_CUDA, "pg_search_layered: event set-up failed"));
+
+    // ---- top level: strict bounds U_0 < U_1 < ... up to cap
+    long long lb = h0;  // C* >= f_min of every failed pass
+    int finished = 0, cstar = -1;
+    LayPassOut top;
+    if (h0 >= cap) { // h(start) >= U: nothing is cheaper than the incumbent
+        finished = 2;
+        lb = cap;
+    }
+    for (long long U = std::min<long long>((long long)h0 + 1, cap); !finished;) {
+        LayPassIn in;
+        memcpy(in.s, origin, sizeof(in.s));
+        memcpy(in.t, goal, sizeof(in.t));
+        in.g0 = 0;
+        in.U = (int)U;
+        in.hist_w = bin_width(U, h0);
+        in.strict = true;
+        in.retain = false;
+        in.mid = D / 2;
+        LAY_CHECK(S.pass(in, top));
+        if (S.st.iterations == 0) S.st.first_bound = (int32_t)U;
+        S.st.iterations++;
+        S.st.last_bound = (int32_t)U;
+        S.st.top_expansions = top.expansions;
+        if (top.reached) {
+            cstar = top.goal_g;
+            finished = 1;
+            lb = cstar;
+            break;
+        }
+        if (top.aborted || (S.out_of_budget && top.levels == 0)) break; // the budget ran out inside (or before) the pass
+        const long long fmin = top.fmin == INT_MAX ? cap : top.fmin;
+        lb = std::max(lb, std::min(fmin, cap));
+        if (fmin >= cap) {
+            if (!has_inc) return finish(pg_fail(ctx, PG_ERR_STATE, "pg_search_layered: no path below the all-advance cost"));
+            finished = 2; // nothing below U = the incumbent's cost: it is optimal
+            lb = cap;
+            break;
+        }
+        if (S.out_of_budget) break;
+        U = next_bound(top, (int)U, in.hist_w, cap);
+    }
+
+    // ---- reconstruction: the top pass's relay splits the alignment, each half solved by narrower passes
+    std::vector<uint32_t> masks;
+    if (finished == 1 && rows) {
+        S.C = cstar;
+        if (retain_all)
+            LAY_CHECK(S.solve(origin, goal, 0, cstar, 1, masks));
+        else
+            LAY_CHECK(S.split(origin, goal, 0, cstar, top, 0, masks));
+        if (S.out_of_budget) {
+            finished = 0; // C* is proved (lower bound == C*), but the alignment is not complete: no rows
+            masks.clear();
+        } else if (pg_path_cost(ctx, masks) != cstar) {
+            return finish(pg_fail(ctx, PG_ERR_STATE, "pg_search_layered: the reconstructed alignment does not cost C*"));
+        }
+    }
+    if (cudaEventRecord(ev1, ctx->stream) != cudaSuccess || cudaEventSynchronize(ev1) != cudaSuccess)
+        return finish(pg_fail(ctx, PG_ERR_CUDA, "pg_search_layered: event failed"));
+    float ms = 0;
+    cudaEventElapsedTime(&ms, ev0, ev1);
+    res->kernel_ms = ms;
+    res->rounds = S.st.levels;
+    res->finished = finished;
+    if (finished == 2) {
+        emit_incumbent(ctx, res, rows);
+    } else if (finished == 1) {
+        res->g = res->f = cstar;
+        if (rows) emit_alignment(ctx, masks, res, rows);
+    }
+    if (finished == 0 && cstar >= 0) lb = cstar;
+    if (has_inc) lb = std::min(lb, (long long)ctx->inc_cost);
+    ctx->lower_bound = (int32_t)lb;
+    ctx->lb_valid = true;
+    S.st.peak_bytes = pg_layered_bytes(S.L);
+    if (stats) *stats = S.st;
+    res->seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+    return finish(PG_OK);
+#undef LAY_CHECK
 }
 
 extern "C" int pg_search_set_weight(pg_ctx *ctx, int32_t num, int32_t den)

@@ -220,6 +220,39 @@ int pg_run_rounds(pg_ctx *ctx, int n, int f_limit, int group, bool allow_graph);
 // g of the alignment spelled by `masks` (origin first) under the context's cost model (Node.cpp:129-152).
 long long pg_path_cost(const pg_ctx *ctx, const std::vector<uint32_t> &masks);
 
+// ---- the level passes of the layered search (pg_layered.cu), driven by pg_search_layered (pg_drivers.cu) ---------------
+struct LayeredState; // level tables, level list, relay band, histogram and control block of one layered search
+constexpr int PG_LAYERED_BINS = 2048; // histogram of the pruned f
+// One pass over the box [s, t] from s with g(s) = g0: keeps the successors with g + h < U (strict) or <= U.  Relay mode
+// (retain == false) holds N + 1 level tables and reports the relay of t; retain mode keeps every level of the box with
+// its parent masks, for pg_layered_trace.
+struct LayPassIn {
+    int s[PG_MAX_SEQ], t[PG_MAX_SEQ];
+    int g0, U;
+    int hist_w;         // width of the histogram's bins
+    bool strict, retain;
+    int mid;            // relay mode: the relay is the first node of t's path above this level
+};
+struct LayPassOut {
+    bool reached = false, aborted = false; // t kept; the expansion budget ran out inside the pass
+    int goal_g = -1;
+    int relay[PG_MAX_SEQ] = {0};           // relay mode: x, the first node above mid on t's path, its g and the move into it
+    int relay_g = 0;
+    uint32_t relay_mask = 0;
+    int fmin = INT_MAX, fmax = INT_MIN;    // over the successors that failed the bound only
+    std::vector<unsigned long long> hist;  // of their f: bin b counts f in [U + b w, U + (b + 1) w), the last bin also
+                                           // everything above
+    int64_t expansions = 0, generated = 0, inserted = 0, levels = 0, max_level_nodes = 0, max_held = 0;
+};
+// retain_levels: the widest box (in levels + 1) a retain pass may cover; level_cap: coordinates one level may hold.
+int pg_layered_open(pg_ctx *ctx, int64_t level_cap, int retain_levels, LayeredState **out);
+void pg_layered_close(pg_ctx *ctx, LayeredState *L);
+int64_t pg_layered_bytes(const LayeredState *L);
+// budget > 0: the pass stops (aborted) once its expansions reach it
+int pg_layered_pass(pg_ctx *ctx, LayeredState *L, const LayPassIn &in, int64_t budget, LayPassOut &out);
+// after a retain pass that reached t: the moves from s to t (s first)
+int pg_layered_trace(pg_ctx *ctx, LayeredState *L, const LayPassIn &in, std::vector<uint32_t> &masks);
+
 // ---- device helpers ------------------------------------------------------------------------
 #ifdef __CUDACC__
 __device__ __forceinline__ int pg_pair_index(int n, int x, int y) // x < y, (i<j) order of HeuristicHPair.cpp:54-61
