@@ -325,6 +325,41 @@ typedef struct {
     int64_t peak_bytes, top_expansions; /* device bytes the mode allocated; expansions of the last top-level pass      */
 } pg_layered_stats;
 int pg_search_layered(pg_ctx *ctx, const pg_search_config *cfg, pg_result *res, pg_layered_stats *stats, char *const *rows);
+/* Breadth-first beam search over the lattice levels (no reference counterpart): the level passes of pg_search_layered,
+ * strict at U, where each level keeps only its W least nodes by (f = g + h, packed key Σ pos_i << (i key_bits)) before it
+ * is expanded.  Kept nodes store their parent, and the alignment is traced back from the goal.  Memory is bounded by W;
+ * the nodes the cut drops certify a lower bound.  One phase per width, each bounded by the best alignment so far, so a
+ * phase that reaches the goal strictly improves it; the loop stops once the lower bound reaches the best cost.
+ * Exact costs with gap_open == gap_ext only.
+ *   widths[0 .. n_widths - 1] (n_widths 1..64, every width >= 1): W of each phase.
+ *   cfg->table_capacity: coordinates the N + 1 level tables hold at once, candidates before the cut (each level at most
+ *                        1 / (N + 1) of it; 0 = (N + 1) x min(the widest lattice level, max(2^16, 64 x the largest W)));
+ *                        a level that does not fit gives PG_ERR_CAPACITY.  cfg->max_expansions (0: none): a budget over
+ *                        all phases.  The other fields are ignored.
+ *   res: finished 1 (a phase found the alignment returned and the lower bound equals its cost), 2 (an alignment with a
+ *        gap to the lower bound, or the incumbent returned unimproved), 0 (no alignment is known).  expansions /
+ *        generated / inserted are summed over the phases, rounds = levels swept, closed_size = nodes kept, open_size =
+ *        nodes dropped by the cut.
+ *   phase_res, phase_lb (may be NULL; n_widths entries): per phase finished (1: it reached the goal), g (-1: not
+ *        reached), the counters as res, and its lower bound min(g, the least f dropped, U); -1 for a phase that did not
+ *        run or that the budget stopped.
+ *   rows (may be NULL): as pg_search.  stats (may be NULL): see pg_beam_stats.
+ * Each phase's LB is a certified lower bound on the optimum; afterwards pg_search_lower_bound gives their maximum (h(start)
+ * when no phase completed).  Honours pg_search_set_incumbent; as pg_search_anytime, a phase that improves the alignment
+ * makes it the context's incumbent, so afterwards the incumbent is the alignment returned.  The retained array holds
+ * sum over levels of min(W, |level|) entries for the largest W: more than 2^32 - 1, or more device memory than is free,
+ * gives PG_ERR_CAPACITY before any device work.  PG_ERR_ARG for a bad width list or a search weight other than 1,
+ * PG_ERR_UNSUPPORTED for gap_open != gap_ext or a key over 127 bits, PG_ERR_STATE without pair tables or while a
+ * step-wise search is active. */
+typedef struct {
+    int32_t phases, best_phase;     /* phases run; the phase whose alignment is returned (-1: none found)              */
+    int64_t levels, kept, dropped;  /* over all phases: levels swept, nodes kept (= expanded), nodes dropped by the cut */
+    int64_t max_candidates;         /* most candidates of one level before the cut                                    */
+    int64_t retained;               /* entries of the retained array                                                  */
+    int64_t peak_bytes;             /* device bytes the mode allocated                                                */
+} pg_beam_stats;
+int pg_search_beam(pg_ctx *ctx, const pg_search_config *cfg, const int64_t *widths, int n_widths, pg_result *res,
+                   pg_result *phase_res, int32_t *phase_lb, pg_beam_stats *stats, char *const *rows);
 /* bytes per exchanged successor record for this context */
 int pg_xrec_stride(const pg_ctx *ctx);
 

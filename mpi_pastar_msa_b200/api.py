@@ -12,6 +12,7 @@ Reference interface                                   -> here
   (no reference counterpart: bounded-suboptimal search) -> .search(weight=W) / .search_set_weight / .search_lower_bound
   (no reference counterpart: incumbent / anytime search) -> .score_alignment / .search(incumbent=rows) / .anytime_search
   (no reference counterpart: layered search)           -> .layered_search
+  (no reference counterpart: beam search)              -> .beam_search
 """
 import ctypes as C
 import math
@@ -53,6 +54,14 @@ class LayeredStats(C.Structure):
     _fields_ = [("iterations", C.c_int32), ("first_bound", C.c_int32), ("last_bound", C.c_int32), ("depth", C.c_int32),
                 ("passes", C.c_int64), ("levels", C.c_int64), ("max_level_nodes", C.c_int64), ("max_held", C.c_int64),
                 ("peak_bytes", C.c_int64), ("top_expansions", C.c_int64)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class BeamStats(C.Structure):
+    _fields_ = [("phases", C.c_int32), ("best_phase", C.c_int32), ("levels", C.c_int64), ("kept", C.c_int64),
+                ("dropped", C.c_int64), ("max_candidates", C.c_int64), ("retained", C.c_int64), ("peak_bytes", C.c_int64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -128,6 +137,8 @@ def load_library():
         "pg_search_anytime": ([vp, C.POINTER(SearchConfig), C.POINTER(C.c_int32), C.POINTER(C.c_int32), i32, C.POINTER(Result),
                                C.POINTER(Result), C.POINTER(C.c_int32), C.POINTER(C.c_char_p)], i32),
         "pg_search_layered": ([vp, C.POINTER(SearchConfig), C.POINTER(Result), C.POINTER(LayeredStats), C.POINTER(C.c_char_p)], i32),
+        "pg_search_beam": ([vp, C.POINTER(SearchConfig), C.POINTER(C.c_int64), i32, C.POINTER(Result), C.POINTER(Result),
+                            C.POINTER(C.c_int32), C.POINTER(BeamStats), C.POINTER(C.c_char_p)], i32),
     }
     for name, (args, res) in sig.items():
         f = getattr(L, name)
@@ -143,7 +154,7 @@ EXPORTS = ["pg_release_cached_memory", "pg_search_note_rounds", "pg_search_set_d
            "pg_owner", "pg_expand_batch", "pg_expand_batch_dev", "pg_search", "pg_search_begin", "pg_search_round",
            "pg_search_outbox", "pg_search_insert_dev", "pg_search_status", "pg_search_lookup", "pg_search_lookup_batch",
            "pg_search_end", "pg_xrec_stride", "pg_search_set_weight", "pg_search_lower_bound", "pg_score_alignment", "pg_search_set_incumbent",
-           "pg_search_anytime", "pg_search_layered"]
+           "pg_search_anytime", "pg_search_layered", "pg_search_beam"]
 
 WEIGHT_DEN = 1024
 
@@ -520,6 +531,30 @@ class PastarGPU:
         if res.finished == 1 and not want_rows:
             d.pop("rows", None)
         d["layered"] = st.as_dict()
+        return d
+
+    def beam_search(self, widths, incumbent=None, table_capacity=0, max_expansions=0, want_rows=True):
+        """pg_search_beam: breadth-first beam search over the lattice levels, one phase per width W (each level keeps its
+        W least nodes by (f, packed key) before it is expanded), each bounded by the best alignment so far (the incumbent,
+        if given, for the first).  table_capacity: coordinates the level tables hold at once, candidates before the cut
+        (0: the default of pg_search_beam); max_expansions: a budget over all phases.  Returns the usual dict (finished 1:
+        proved optimal, 2: an alignment with a gap to lower_bound or the incumbent unimproved, 0: none) with
+        `lower_bound`, `phases`, one dict per phase that completed (width, g (-1: the goal was not reached), lower_bound,
+        expansions, kept, dropped), and `beam`, the statistics (pg_beam_stats)."""
+        if incumbent is not None:
+            self.search_set_incumbent(incumbent)
+        widths = [int(w) for w in widths]
+        k = len(widths)
+        ws = (C.c_int64 * max(k, 1))(*widths)
+        cfg = SearchConfig(1, 0, table_capacity, 0, max_expansions, 0, 0)
+        res, pres, plb, st = Result(), (Result * max(k, 1))(), (C.c_int32 * max(k, 1))(), BeamStats()
+        rows, bufs = self._row_bufs(want_rows)
+        self._ck(self.L.pg_search_beam(self.h, C.byref(cfg), ws, k, C.byref(res), pres, plb, C.byref(st), rows))
+        d = self._result(res, bufs)
+        d["phases"] = [{"width": widths[i], "g": pres[i].g, "lower_bound": plb[i], "expansions": pres[i].expansions,
+                        "generated": pres[i].generated, "inserted": pres[i].inserted, "levels": pres[i].rounds,
+                        "kept": pres[i].closed_size, "dropped": pres[i].open_size} for i in range(k) if plb[i] >= 0]
+        d["beam"] = st.as_dict()
         return d
 
     def search_lower_bound(self):

@@ -412,6 +412,8 @@ struct PAStarOpt { // PAStar.h:87-112, plus the GPU-side knobs (new, do not chan
     std::vector<std::string> incumbent_rows; // its rows, checked against the input before any device call
     std::vector<int32_t> anytime_num;        // --anytime W1,W2,...: one weighted phase per weight, num / 1024 (empty: not given)
     bool layered = false;                    // --layered: pg_search_layered instead of pg_search (one GPU, exact)
+    std::vector<int64_t> beam_widths;        // --beam W1,W2,...: pg_search_beam, one phase per width (empty: not given);
+                                             // with --layered its alignment is the layered search's incumbent
 };
 
 int read_fasta_file(const std::string &name);
@@ -450,9 +452,17 @@ class PAStar {
         for (int i = 0; i < N; i++) rowp[i] = bufs[i].data();
         const int wden = 1024;
         int32_t lower_bound = 0;
-        const bool bounded = options.weight_num || !options.incumbent_rows.empty() || !options.anytime_num.empty() || options.layered;
+        const int n_beam = (int)options.beam_widths.size();
+        const bool bounded = options.weight_num || !options.incumbent_rows.empty() || !options.anytime_num.empty() || options.layered || n_beam;
         pg_layered_stats lst;
         memset(&lst, 0, sizeof(lst));
+        pg_beam_stats bst;
+        memset(&bst, 0, sizeof(bst));
+        std::vector<pg_result> beam_res(n_beam);
+        std::vector<int32_t> beam_lb(n_beam, -1);
+        pg_result beam_total;
+        memset(&beam_total, 0, sizeof(beam_total));
+        int32_t beam_bound = 0;
         std::vector<const char *> inc(N);
         for (int i = 0; i < (int)options.incumbent_rows.size(); i++) inc[i] = options.incumbent_rows[i].c_str();
         const int inc_cols = options.incumbent_rows.empty() ? 0 : (int)options.incumbent_rows[0].size();
@@ -465,6 +475,13 @@ class PAStar {
             if (options.weight_num) h->check(pg_search_set_weight(h->ctx, options.weight_num, wden), "pg_search_set_weight");
             if (inc_cols) h->check(pg_search_set_incumbent(h->ctx, inc.data(), inc_cols), "pg_search_set_incumbent");
             TimeCounter t("Phase 2: PA-Star running time: ");
+            if (n_beam) { // its best alignment is the context's incumbent afterwards: it bounds --layered
+                h->check(pg_search_beam(h->ctx, &cfg, options.beam_widths.data(), n_beam, &beam_total, beam_res.data(), beam_lb.data(),
+                                        &bst, rowp.data()),
+                         "pg_search_beam");
+                h->check(pg_search_lower_bound(h->ctx, &beam_bound), "pg_search_lower_bound");
+                res = beam_total;
+            }
             if (n_phases) {
                 const std::vector<int32_t> dens(n_phases, wden);
                 h->check(pg_search_anytime(h->ctx, &cfg, options.anytime_num.data(), dens.data(), n_phases, &res, phase_res.data(),
@@ -472,7 +489,7 @@ class PAStar {
                          "pg_search_anytime");
             } else if (options.layered) {
                 h->check(pg_search_layered(h->ctx, &cfg, &res, &lst, rowp.data()), "pg_search_layered");
-            } else {
+            } else if (!n_beam) {
                 h->check(pg_search(h->ctx, &cfg, &res, rowp.data()), "pg_search");
             }
             parts[0] = res;
@@ -492,7 +509,7 @@ class PAStar {
         // weighted, incumbent-bounded and anytime search: the optimum is at least the lower bound, so g / bound is the
         // certified ratio to it (1: the alignment is proved optimal)
         auto print_bound = [&]() {
-            if (!(options.weight_num > wden || inc_cols || n_phases || options.layered)) return;
+            if (!(options.weight_num > wden || inc_cols || n_phases || options.layered || n_beam)) return;
             std::cout << "Lower bound: " << lower_bound;
             if (res.finished) std::cout << "\tg / lower bound: " << std::fixed << std::setprecision(4) << (double)res.g / lower_bound;
             std::cout << std::endl;
@@ -506,6 +523,13 @@ class PAStar {
                           << "), " << lst.passes << " passes, " << lst.levels << " levels, depth " << lst.depth << ", widest level "
                           << lst.max_level_nodes << ", at most " << lst.max_held << " coordinates held, " << lst.peak_bytes
                           << " bytes" << std::endl;
+            if (n_beam) {
+                std::cout << "Beam: score " << beam_total.g << ", lower bound " << beam_bound << ";";
+                for (int k = 0; k < n_beam; k++)
+                    if (beam_lb[k] >= 0)
+                        std::cout << " width " << options.beam_widths[k] << ": score " << beam_res[k].g << ", lower bound " << beam_lb[k] << ";";
+                std::cout << " " << bst.kept << " kept, " << bst.dropped << " dropped, " << bst.peak_bytes << " bytes" << std::endl;
+            }
         };
         if (!res.finished) {
             std::cout << "Search stopped at the expansion budget: " << res.expansions << " expansions, no alignment.\n";
@@ -566,6 +590,21 @@ class PAStar {
                    << ", \"last_bound\": " << lst.last_bound << ", \"depth\": " << lst.depth << ", \"passes\": " << lst.passes
                    << ", \"levels\": " << lst.levels << ", \"max_level_nodes\": " << lst.max_level_nodes << ", \"max_held\": "
                    << lst.max_held << ", \"peak_bytes\": " << lst.peak_bytes << ", \"top_expansions\": " << lst.top_expansions << "}";
+            if (n_beam) {
+                js << ", \"beam\": {\"g\": " << beam_total.g << ", \"finished\": " << beam_total.finished << ", \"lower_bound\": " << beam_bound
+                   << ", \"phases\": [";
+                bool first = true;
+                for (int k = 0; k < n_beam; k++) {
+                    if (beam_lb[k] < 0) continue;
+                    js << (first ? "" : ", ") << "{\"width\": " << options.beam_widths[k] << ", \"g\": " << beam_res[k].g
+                       << ", \"lower_bound\": " << beam_lb[k] << ", \"expansions\": " << beam_res[k].expansions << ", \"kept\": "
+                       << beam_res[k].closed_size << ", \"dropped\": " << beam_res[k].open_size << "}";
+                    first = false;
+                }
+                js << "], \"best_phase\": " << bst.best_phase << ", \"levels\": " << bst.levels << ", \"kept\": " << bst.kept
+                   << ", \"dropped\": " << bst.dropped << ", \"max_candidates\": " << bst.max_candidates << ", \"retained\": "
+                   << bst.retained << ", \"peak_bytes\": " << bst.peak_bytes << "}";
+            }
             js << ", \"total\": ";
             one(res);
             js << ", \"partitions\": [";

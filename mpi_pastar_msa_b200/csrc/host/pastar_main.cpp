@@ -2,7 +2,7 @@
 //
 //   pastar [-t N] [-s SHIFT] [-y FZORDER|FSUM|PZORDER|PSUM] [-v] [-h] [--memory_debug] file.fasta
 //   new, optional: [-g/--gpus N] [--batch K] [--table_capacity SLOTS] [--max_expansions E] [--metrics_json FILE] [--weight W]
-//                  [--incumbent FILE] [--anytime W1,W2,...] [--layered]
+//                  [--incumbent FILE] [--anytime W1,W2,...] [--layered] [--beam W1,W2,...]
 //
 // Same flags, exit codes (0 ok, 1 usage / not a regular file, -1 on exception) and stdout format as the reference
 // (phase timers, "Final Score:", "Similarity:", wrapped alignment, "Total nodes count:" table).  No MPI: the
@@ -72,6 +72,9 @@ static void usage(const char *argv0)
               << "                                by the best alignment so far (one GPU)\n"
               << "  --layered                     exact search level by level: holds a few lattice levels, not every\n"
               << "                                coordinate generated (one GPU; composes with --incumbent)\n"
+              << "  --beam arg                    comma-separated beam widths (at most 64): breadth-first beam search,\n"
+              << "                                one phase per width, each bounded by the best alignment so far (one\n"
+              << "                                GPU; composes with --incumbent, and seeds --layered)\n"
               << std::endl;
 }
 
@@ -94,7 +97,7 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
     // Boost.ProgramOptions' default style lets a long option be shortened to any unambiguous prefix ("--thr 4", "--hash_t=FSUM")
     static const char *const long_names[] = {"version", "help", "memory_debug", "threads", "hash_shift", "hash_type", "gpus",
                                              "batch", "table_capacity", "max_expansions", "metrics_json", "weight",
-                                             "incumbent", "anytime", "layered"};
+                                             "incumbent", "anytime", "layered", "beam"};
     auto canonical = [&](const std::string &arg) -> std::string {
         if (arg.size() < 3 || arg.compare(0, 2, "--") != 0) return arg;
         const size_t eq = arg.find('=');
@@ -150,6 +153,27 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
             }
             if (opt.anytime_num.size() > 64) throw std::invalid_argument("the argument for option '--anytime' has more than 64 weights");
         }
+        else if (is_long(a, "beam")) {
+            const std::string v = value(i, a, "beam");
+            opt.beam_widths.clear();
+            for (size_t at = 0;;) {
+                const size_t comma = v.find(',', at);
+                const std::string w = v.substr(at, comma == std::string::npos ? std::string::npos : comma - at);
+                size_t used = 0;
+                long long x = 0;
+                try {
+                    x = std::stoll(w, &used);
+                } catch (const std::exception &) {
+                    used = 0;
+                }
+                if (w.empty() || used != w.size() || x < 1)
+                    throw std::invalid_argument("the argument for option '--beam' must be positive integers separated by commas");
+                opt.beam_widths.push_back(x);
+                if (comma == std::string::npos) break;
+                at = comma + 1;
+            }
+            if (opt.beam_widths.size() > 64) throw std::invalid_argument("the argument for option '--beam' has more than 64 widths");
+        }
         else if (!a.empty() && a[0] == '-' && a.size() > 1) throw std::invalid_argument("unrecognised option '" + a + "'");
         else {
             filename = a; // file.fasta is position independent
@@ -167,6 +191,10 @@ static int options_core(int argc, char *argv[], std::string &filename, PAStarOpt
     if (opt.layered && opt.weight_num && opt.weight_num != 1024)
         throw std::invalid_argument("option '--layered' cannot be combined with '--weight' other than 1");
     if (opt.layered && opt.gpus != 1) throw std::invalid_argument("option '--layered' cannot be combined with '--gpus' above 1");
+    if (!opt.beam_widths.empty() && !opt.anytime_num.empty()) throw std::invalid_argument("option '--beam' cannot be combined with '--anytime'");
+    if (!opt.beam_widths.empty() && opt.weight_num && opt.weight_num != 1024)
+        throw std::invalid_argument("option '--beam' cannot be combined with '--weight' other than 1");
+    if (!opt.beam_widths.empty() && opt.gpus != 1) throw std::invalid_argument("option '--beam' cannot be combined with '--gpus' above 1");
     if (version) {
         std::cout << "msa_pastar, version 1.0\n";
         std::exit(0);

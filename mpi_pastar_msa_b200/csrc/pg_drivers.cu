@@ -1,6 +1,8 @@
 // Host drivers of the search (no kernels): whole searches built on the step-wise machinery of pg_search.cu.
 //   pg_search          one partition on one GPU, rounds in groups replayed as CUDA graphs
 //   pg_search_anytime  weighted searches with falling weights, each bounded by the best alignment so far
+//   pg_search_layered  breadth-first heuristic search level by level (the level passes are in pg_layered.cu)
+//   pg_search_beam     breadth-first beam search over the same level passes, one phase per width
 //   pg_multi_search    the hash-partitioned search over the GPUs of one box, one host thread per GPU
 // plus what they share: alignment scoring and the incumbent, the search weight, the lower bound and the result.
 #include <algorithm>
@@ -254,6 +256,31 @@ long long move_cost(const pg_ctx *ctx, const int *pos, uint32_t m)
     return sum;
 }
 
+// The refusals shared by the level-pass searches (pg_search_layered, pg_search_beam)
+int level_search_refusals(pg_ctx *ctx, const char *fn)
+{
+    int rc = refuse_while_stepwise(ctx, fn);
+    if (rc != PG_OK) return rc;
+    if (!ctx->tables_built) return pg_fail(ctx, PG_ERR_STATE, std::string(fn) + ": pg_build_pair_tables has not run");
+    if (ctx->dp.gap_open != ctx->dp.gap_ext)
+        return pg_fail(ctx, PG_ERR_UNSUPPORTED, std::string(fn) + ": gap_open != gap_ext (a coordinate is then not a state)");
+    if (ctx->wnum != 1 || ctx->wsh != 0) return pg_fail(ctx, PG_ERR_ARG, std::string(fn) + ": exact search only (search weight 1)");
+    if (ctx->n * ctx->dp.key_bits > 127) return pg_fail(ctx, PG_ERR_UNSUPPORTED, "packed coordinate key exceeds 127 bits");
+    return PG_OK;
+}
+
+// cost of the alignment whose column c advances every sequence longer than c: the search's UB, as pg_search_begin
+long long all_advance_cost(const pg_ctx *ctx)
+{
+    std::vector<uint32_t> all_advance;
+    for (int c = 0, mx = *std::max_element(ctx->len, ctx->len + ctx->n); c < mx; c++) {
+        uint32_t m = 0;
+        for (int i = 0; i < ctx->n; i++) m |= (uint32_t)(c < ctx->len[i]) << i;
+        all_advance.push_back(m);
+    }
+    return pg_path_cost(ctx, all_advance);
+}
+
 // Bin width of a top-level pass at bound U: the bins below the last one span 2 (U - h(start)), so the bound can at most
 // triple its distance from h(start) in one step.
 int bin_width(long long U, long long h0)
@@ -359,13 +386,8 @@ struct Layered {
 extern "C" int pg_search_layered(pg_ctx *ctx, const pg_search_config *cfg_in, pg_result *res, pg_layered_stats *stats, char *const *rows)
 {
     if (!ctx || !res) return PG_ERR_ARG;
-    int rc = refuse_while_stepwise(ctx, "pg_search_layered");
+    int rc = level_search_refusals(ctx, "pg_search_layered");
     if (rc != PG_OK) return rc;
-    if (!ctx->tables_built) return pg_fail(ctx, PG_ERR_STATE, "pg_search_layered: pg_build_pair_tables has not run");
-    if (ctx->dp.gap_open != ctx->dp.gap_ext)
-        return pg_fail(ctx, PG_ERR_UNSUPPORTED, "pg_search_layered: gap_open != gap_ext (a coordinate is then not a state)");
-    if (ctx->wnum != 1 || ctx->wsh != 0) return pg_fail(ctx, PG_ERR_ARG, "pg_search_layered: exact search only (search weight 1)");
-    if (ctx->n * ctx->dp.key_bits > 127) return pg_fail(ctx, PG_ERR_UNSUPPORTED, "packed coordinate key exceeds 127 bits");
     const pg_search_config cfg = config_or_zero(cfg_in);
     if (cfg.table_capacity < 0 || cfg.max_expansions < 0) return pg_fail(ctx, PG_ERR_ARG, "pg_search_layered: negative capacity or budget");
     PG_CUDA(ctx, cudaSetDevice(ctx->device));
@@ -382,13 +404,7 @@ extern "C" int pg_search_layered(pg_ctx *ctx, const pg_search_config *cfg_in, pg
     std::vector<uint16_t> zero(n, 0);
     int32_t h0 = 0;
     if ((rc = pg_calculate_h(ctx, zero.data(), 1, &h0)) != PG_OK) return rc;
-    std::vector<uint32_t> all_advance; // the search's UB, as pg_search_begin
-    for (int c = 0, mx = *std::max_element(ctx->len, ctx->len + n); c < mx; c++) {
-        uint32_t m = 0;
-        for (int i = 0; i < n; i++) m |= (uint32_t)(c < ctx->len[i]) << i;
-        all_advance.push_back(m);
-    }
-    const long long ub = pg_path_cost(ctx, all_advance);
+    const long long ub = all_advance_cost(ctx);
     const bool has_inc = ctx->inc_cost >= 0;
     const long long cap = has_inc ? ctx->inc_cost : ub + 1; // strict bounds: the last pass keeps g + h < cap
     if (cap > INT_MAX - 1) return pg_fail(ctx, PG_ERR_UNSUPPORTED, "pg_search_layered: the upper bound does not fit 31 bits");
@@ -402,7 +418,7 @@ extern "C" int pg_search_layered(pg_ctx *ctx, const pg_search_config *cfg_in, pg
     S.retain_levels = retain_all ? D + 1 : (deep ? 1 : 4 * (n + 1));
     S.budget = cfg.max_expansions;
     const int64_t capacity = cfg.table_capacity > 0 ? cfg.table_capacity : (1LL << 22);
-    if ((rc = pg_layered_open(ctx, std::max<int64_t>(1, capacity / (n + 1)), S.retain_levels, &S.L)) != PG_OK) {
+    if ((rc = pg_layered_open(ctx, std::max<int64_t>(1, capacity / (n + 1)), S.retain_levels, 0, &S.L)) != PG_OK) {
         pg_layered_close(ctx, S.L);
         return rc;
     }
@@ -500,6 +516,189 @@ extern "C" int pg_search_layered(pg_ctx *ctx, const pg_search_config *cfg_in, pg
     res->seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     return finish(PG_OK);
 #undef LAY_CHECK
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// pg_search_beam: breadth-first beam search over the lattice levels: strict level passes under the best alignment so far
+// that keep the W least (f, packed key) of every level, one phase per width.  The cut is in pg_layered.cu; DESIGN.md §4.4d.
+// ---------------------------------------------------------------------------------------------------------------------
+namespace {
+
+// Coordinates of the lattice on each level 0 .. D: the coefficients of prod_i (1 + x + ... + x^len_i), saturated at 2^62.
+// Every coefficient is capped at 2^100 before the window sums, so a window that holds a capped term is itself >= 2^100.
+std::vector<int64_t> level_sizes(const pg_ctx *ctx)
+{
+    typedef unsigned __int128 u128;
+    const u128 CAP = (u128)1 << 100;
+    std::vector<u128> c(1, 1);
+    for (int i = 0; i < ctx->n; i++) {
+        const size_t L = (size_t)ctx->len[i];
+        std::vector<u128> pre(c.size() + 1, 0), nc(c.size() + L);
+        for (size_t d = 0; d < c.size(); d++) pre[d + 1] = pre[d] + c[d];
+        for (size_t d = 0; d < nc.size(); d++) {
+            const size_t hi = std::min(d + 1, c.size()), lo = d >= L ? d - L : 0;
+            nc[d] = std::min(CAP, pre[hi] - pre[lo]);
+        }
+        c.swap(nc);
+    }
+    std::vector<int64_t> out(c.size());
+    for (size_t d = 0; d < c.size(); d++) out[d] = (int64_t)std::min(c[d], (u128)1 << 62);
+    return out;
+}
+
+} // namespace
+
+extern "C" int pg_search_beam(pg_ctx *ctx, const pg_search_config *cfg_in, const int64_t *widths, int n_widths, pg_result *res,
+                              pg_result *phase_res, int32_t *phase_lb, pg_beam_stats *stats, char *const *rows)
+{
+    if (!ctx || !res || !widths) return PG_ERR_ARG;
+    if (n_widths < 1 || n_widths > 64) return pg_fail(ctx, PG_ERR_ARG, "pg_search_beam: n_widths must be in 1..64");
+    for (int k = 0; k < n_widths; k++)
+        if (widths[k] <= 0) return pg_fail(ctx, PG_ERR_ARG, "pg_search_beam: width " + std::to_string(k) + " is not positive");
+    int rc = level_search_refusals(ctx, "pg_search_beam");
+    if (rc != PG_OK) return rc;
+    const pg_search_config cfg = config_or_zero(cfg_in);
+    if (cfg.table_capacity < 0 || cfg.max_expansions < 0) return pg_fail(ctx, PG_ERR_ARG, "pg_search_beam: negative capacity or budget");
+    const int n = ctx->n;
+    int origin[PG_MAX_SEQ] = {0}, goal[PG_MAX_SEQ] = {0}, D = 0;
+    for (int i = 0; i < n; i++) {
+        goal[i] = ctx->len[i];
+        D += ctx->len[i];
+    }
+    const long long ub = all_advance_cost(ctx);
+    if (ctx->inc_cost < 0 && ub + 1 > INT_MAX - 1)
+        return pg_fail(ctx, PG_ERR_UNSUPPORTED, "pg_search_beam: the upper bound does not fit 31 bits");
+
+    // memory: the retained array holds at most min(W, |level d|) nodes of every level expanded; the N + 1 level tables
+    // hold the candidates before the cut, by default 64 W per level (at least 2^16), never more than the widest level
+    const std::vector<int64_t> sizes = level_sizes(ctx);
+    const int64_t wmax = *std::max_element(widths, widths + n_widths);
+    unsigned __int128 retained = 0;
+    for (int d = 0; d < D; d++) retained += (unsigned __int128)std::min(wmax, sizes[d]);
+    if (retained > 0xffffffffu)
+        return pg_fail(ctx, PG_ERR_CAPACITY, "pg_search_beam: the widest beam retains more than 2^32 - 1 nodes");
+    const int64_t widest = *std::max_element(sizes.begin(), sizes.end());
+    const int64_t level_cap = cfg.table_capacity > 0 ? std::max<int64_t>(1, cfg.table_capacity / (n + 1))
+                                                     : std::min(widest, std::max<int64_t>(1LL << 16, 64 * std::min<int64_t>(wmax, 1LL << 40)));
+
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
+    memset(res, 0, sizeof(*res));
+    res->g = res->f = -1;
+    for (int k = 0; k < n_widths; k++) {
+        if (phase_res) {
+            memset(&phase_res[k], 0, sizeof(pg_result));
+            phase_res[k].g = phase_res[k].f = -1;
+        }
+        if (phase_lb) phase_lb[k] = -1;
+    }
+    pg_beam_stats st;
+    memset(&st, 0, sizeof(st));
+    st.best_phase = -1;
+    st.retained = (int64_t)retained;
+    ctx->lb_valid = false;
+    const auto t0 = std::chrono::steady_clock::now();
+    std::vector<uint16_t> zero(n, 0);
+    int32_t h0 = 0;
+    if ((rc = pg_calculate_h(ctx, zero.data(), 1, &h0)) != PG_OK) return rc;
+
+    LayeredState *L = nullptr;
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    auto finish = [&](int code) {
+        if (ev0) cudaEventDestroy(ev0);
+        if (ev1) cudaEventDestroy(ev1);
+        pg_layered_close(ctx, L);
+        return code;
+    };
+    if ((rc = pg_layered_open(ctx, level_cap, 0, (int64_t)retained, &L)) != PG_OK) return finish(rc);
+    if (cudaEventCreate(&ev0) != cudaSuccess || cudaEventCreate(&ev1) != cudaSuccess || cudaEventRecord(ev0, ctx->stream) != cudaSuccess)
+        return finish(pg_fail(ctx, PG_ERR_CUDA, "pg_search_beam: event set-up failed"));
+
+    size_t total = 1;
+    for (int i = 0; i < n; i++) total += (size_t)ctx->len[i];
+    std::vector<std::vector<char>> bufs(n, std::vector<char>(total));
+    std::vector<char *> rowp(n);
+    for (int i = 0; i < n; i++) rowp[i] = bufs[i].data();
+    bool improved = false, any = false;
+    long long lb = h0; // the maximum over the phases of their certified bounds
+    for (int k = 0; k < n_widths; k++) {
+        const bool has_best = ctx->inc_cost >= 0;
+        if (has_best && lb >= ctx->inc_cost) break; // the best alignment is proved optimal
+        if (cfg.max_expansions > 0 && res->expansions >= cfg.max_expansions) break;
+        LayPassIn in;
+        memcpy(in.s, origin, sizeof(in.s));
+        memcpy(in.t, goal, sizeof(in.t));
+        in.g0 = 0;
+        in.U = (int)(has_best ? ctx->inc_cost : ub + 1);
+        in.hist_w = 1;
+        in.strict = true;
+        in.retain = false;
+        in.mid = D; // no crossing level: every successor carries its parent's retained index
+        in.width = widths[k];
+        LayPassOut o;
+        if ((rc = pg_layered_pass(ctx, L, in, cfg.max_expansions > 0 ? cfg.max_expansions - res->expansions : 0, o)) != PG_OK) {
+            // as pg_search_anytime: a phase that runs out of table ends the loop, and the best alignment so far stands
+            if (rc == PG_ERR_CAPACITY && any) rc = PG_OK;
+            break;
+        }
+        st.phases++;
+        st.levels += o.levels;
+        st.kept += o.kept;
+        st.dropped += o.dropped;
+        st.max_candidates = std::max(st.max_candidates, o.max_cand);
+        res->expansions += o.expansions;
+        res->generated += o.generated;
+        res->inserted += o.inserted;
+        res->rounds += o.levels;
+        res->closed_size += o.kept;
+        res->open_size += o.dropped;
+        if (phase_res) {
+            pg_result &pr = phase_res[k];
+            pr.finished = o.reached && !o.aborted;
+            pr.g = pr.f = pr.finished ? o.goal_g : -1;
+            pr.expansions = o.expansions;
+            pr.generated = o.generated;
+            pr.inserted = o.inserted;
+            pr.rounds = o.levels;
+            pr.closed_size = o.kept;
+            pr.open_size = o.dropped;
+        }
+        if (o.aborted) break; // the budget ran out inside the phase: it certifies nothing
+        // LB: the first node of an optimal path that was not kept was dropped by the cut (f <= C*) or pruned by the
+        // bound (U <= C*); when there is none, the goal was reached with g = C*
+        long long plb = std::min<long long>(in.U, o.drop_fmin);
+        if (o.reached) plb = std::min<long long>(plb, o.goal_g);
+        lb = std::max(lb, plb);
+        any = true;
+        if (phase_lb) phase_lb[k] = (int32_t)plb;
+        if (o.reached) { // g < U: a strict improvement, the next phases' incumbent
+            std::vector<uint32_t> masks;
+            if ((rc = pg_beam_trace(ctx, L, in, o.goal_parent, masks)) != PG_OK) return finish(rc);
+            if (pg_path_cost(ctx, masks) != o.goal_g)
+                return finish(pg_fail(ctx, PG_ERR_STATE, "pg_search_beam: the traced alignment does not cost the goal's g"));
+            pg_result tmp;
+            memset(&tmp, 0, sizeof(tmp));
+            emit_alignment(ctx, masks, &tmp, rowp.data());
+            if ((rc = pg_search_set_incumbent(ctx, rowp.data(), (int32_t)masks.size())) != PG_OK) return finish(rc);
+            improved = true;
+            st.best_phase = k;
+        }
+    }
+    if (rc != PG_OK) return finish(rc);
+    if (cudaEventRecord(ev1, ctx->stream) != cudaSuccess || cudaEventSynchronize(ev1) != cudaSuccess)
+        return finish(pg_fail(ctx, PG_ERR_CUDA, "pg_search_beam: event failed"));
+    float ms = 0;
+    cudaEventElapsedTime(&ms, ev0, ev1);
+    res->kernel_ms = ms;
+    if (ctx->inc_cost >= 0) {
+        emit_incumbent(ctx, res, rows);
+        res->finished = improved && lb >= ctx->inc_cost ? 1 : 2;
+    }
+    ctx->lower_bound = (int32_t)lb;
+    ctx->lb_valid = true;
+    st.peak_bytes = pg_layered_bytes(L);
+    if (stats) *stats = st;
+    res->seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+    return finish(PG_OK);
 }
 
 extern "C" int pg_search_set_weight(pg_ctx *ctx, int32_t num, int32_t den)

@@ -225,13 +225,15 @@ struct LayeredState; // level tables, level list, relay band, histogram and cont
 constexpr int PG_LAYERED_BINS = 2048; // histogram of the pruned f
 // One pass over the box [s, t] from s with g(s) = g0: keeps the successors with g + h < U (strict) or <= U.  Relay mode
 // (retain == false) holds N + 1 level tables and reports the relay of t; retain mode keeps every level of the box with
-// its parent masks, for pg_layered_trace.
+// its parent masks, for pg_layered_trace.  Beam mode (width > 0, relay mode with mid = level(t), tables opened with a
+// retained array) keeps the `width` least (f, packed key) of every level before it is expanded, for pg_beam_trace.
 struct LayPassIn {
     int s[PG_MAX_SEQ], t[PG_MAX_SEQ];
     int g0, U;
     int hist_w;         // width of the histogram's bins
     bool strict, retain;
     int mid;            // relay mode: the relay is the first node of t's path above this level
+    int64_t width = 0;  // beam mode: nodes kept per level (0: no cut)
 };
 struct LayPassOut {
     bool reached = false, aborted = false; // t kept; the expansion budget ran out inside the pass
@@ -243,15 +245,24 @@ struct LayPassOut {
     std::vector<unsigned long long> hist;  // of their f: bin b counts f in [U + b w, U + (b + 1) w), the last bin also
                                            // everything above
     int64_t expansions = 0, generated = 0, inserted = 0, levels = 0, max_level_nodes = 0, max_held = 0;
+    // beam mode: t's parent in the retained array; nodes kept (= retained) and dropped by the cut, the most candidates of
+    // one level before it, the least f dropped
+    uint32_t goal_parent = ~0u;
+    int64_t kept = 0, dropped = 0, max_cand = 0;
+    int drop_fmin = INT_MAX;
 };
-// retain_levels: the widest box (in levels + 1) a retain pass may cover; level_cap: coordinates one level may hold.
-int pg_layered_open(pg_ctx *ctx, int64_t level_cap, int retain_levels, LayeredState **out);
+// retain_levels: the widest box (in levels + 1) a retain pass may cover; level_cap: coordinates one level may hold;
+// beam_retained > 0: beam mode, a retained array of that many entries and no relay band (PG_ERR_CAPACITY when it all
+// needs more bytes than the device has free).
+int pg_layered_open(pg_ctx *ctx, int64_t level_cap, int retain_levels, int64_t beam_retained, LayeredState **out);
 void pg_layered_close(pg_ctx *ctx, LayeredState *L);
 int64_t pg_layered_bytes(const LayeredState *L);
 // budget > 0: the pass stops (aborted) once its expansions reach it
 int pg_layered_pass(pg_ctx *ctx, LayeredState *L, const LayPassIn &in, int64_t budget, LayPassOut &out);
 // after a retain pass that reached t: the moves from s to t (s first)
 int pg_layered_trace(pg_ctx *ctx, LayeredState *L, const LayPassIn &in, std::vector<uint32_t> &masks);
+// after a beam pass that reached t: the moves from s to t (s first) along the retained parents from t's
+int pg_beam_trace(pg_ctx *ctx, LayeredState *L, const LayPassIn &in, uint32_t goal_parent, std::vector<uint32_t> &masks);
 
 // ---- device helpers ------------------------------------------------------------------------
 #ifdef __CUDACC__

@@ -14,6 +14,13 @@
 //
 // A pass is the same three launches per level (compact, expand, advance): the level index and every counter live in the
 // device control block, so a group of levels is captured once as a CUDA graph and replayed.
+//
+// Beam mode (width W > 0, pg_search_beam) is a relay-mode pass over the whole lattice with no crossing level: compaction
+// writes the level's candidates to a staging list, and a cut between compaction and expansion keeps the W least by
+// (f, packed key).  The cut is a radix select decided on the device (score, one launch per 8-bit digit of f - f_min and of
+// the key, keep), so the launches of a level stay the same and replay as a graph.  Each kept node is appended to the
+// retained array as {key, g << 32 | parent's retained index}, and its low in the expand list is its own retained index,
+// so every successor carries its parent's index and the alignment is traced back from the goal's.
 #include <algorithm>
 #include <climits>
 #include <cstring>
@@ -41,6 +48,20 @@ struct LayCtrl {
     uint32_t relay_n;    // relay entries saved
     uint32_t pad;
     unsigned long long expansions, generated, inserted, levels, max_level, max_held;
+    // beam mode: the cut of level d
+    uint32_t cand_n;             // candidates of level d before the cut
+    uint32_t sel_all;            // 1: cand_n <= width, every candidate is kept
+    uint32_t sel_done;           // 1: the kept set is decided
+    uint32_t sel_k;              // candidates still to take from the tie class of the prefix
+    uint32_t blocks_done;        // last-block handshake of the score and select kernels
+    uint32_t keep_n;             // kept entries written so far
+    int32_t lvl_fmin, lvl_fmax;  // f range of level d (score kernel accumulators)
+    int32_t sel_f0;              // level d's least f: the select orders by the unsigned f - sel_f0, then the key
+    uint32_t sel_fp, sel_fm;     // decided bits of f - sel_f0: prefix and mask
+    int32_t drop_fmin;           // least f of the candidates the cut dropped
+    unsigned long long sel_kp[2], sel_km[2]; // decided bits of the packed key (lo, hi word)
+    unsigned long long ret_base, ret_n;      // first retained index of level d; retained entries so far
+    unsigned long long dropped, max_cand;
 };
 
 struct DevLay {
@@ -65,6 +86,16 @@ struct DevLay {
     int hist_w;
     unsigned long long *hist;
     LayCtrl *ctrl;
+    // beam mode
+    uint32_t width;                // 0: no cut
+    int kd;                        // 8-bit digits of the packed key: ceil(n kb / 8)
+    unsigned long long *cand_key;  // KEYW x L, word-major: the level before the cut
+    unsigned long long *cand_val;
+    int32_t *cand_f;               // f of each candidate
+    uint32_t *sel_hist;            // 256 bins of the select pass
+    unsigned long long *ret_key;   // KEYW x ret_cap, word-major
+    unsigned long long *ret_val;   // g << 32 | the parent's retained index (~0: the origin)
+    unsigned long long ret_cap;
 };
 
 __device__ __forceinline__ int lay_table(const DevLay &d, int level) { return d.retain ? level - d.ls : level % d.nt; }
@@ -159,16 +190,16 @@ __device__ __forceinline__ Key<KEYW> lay_pos_key(const DevLay &d, const int *pos
     return k;
 }
 
-// s enters its level's table with g0; the control block starts the pass at level(s)
+// s enters its level's table with g0 and low0; the control block starts the pass at level(s)
 template <int KEYW>
-__global__ void layered_seed_kernel(const __grid_constant__ DevLay d, int g0)
+__global__ void layered_seed_kernel(const __grid_constant__ DevLay d, int g0, uint32_t low0)
 {
     LayCtrl *c = d.ctrl;
     c->d = d.ls;
-    c->fmin = INT_MAX;
-    c->fmax = INT_MIN;
+    c->fmin = c->lvl_fmin = c->drop_fmin = INT_MAX;
+    c->fmax = c->lvl_fmax = INT_MIN;
     const Key<KEYW> k = lay_pos_key<KEYW>(d, d.s);
-    lay_insert<KEYW>(d, d.ls, k, ((unsigned long long)(unsigned)g0 << 32) | (d.retain ? (1u << d.n) - 1u : RELAY_BASE));
+    lay_insert<KEYW>(d, d.ls, k, ((unsigned long long)(unsigned)g0 << 32) | low0);
     c->inserted = 1;
 }
 
@@ -375,6 +406,243 @@ __global__ void layered_trace_kernel(const __grid_constant__ DevLay d, uint32_t 
     out[0] = ~0u;
 }
 
+// ---- beam mode: the cut of level d ----------------------------------------------------------------------------------
+
+template <int KEYW>
+__device__ __forceinline__ Key<KEYW> beam_cand_key(const DevLay &d, uint32_t i)
+{
+    Key<KEYW> k;
+    k.lo = d.cand_key[i];
+    if constexpr (KEYW == 2) k.hi = d.cand_key[d.L + i];
+    return k;
+}
+
+// true in every thread of the last block of the grid to get here; the other blocks' atomics are then visible
+__device__ __forceinline__ bool beam_last_block(LayCtrl *c)
+{
+    __shared__ bool last;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        last = atomicAdd(&c->blocks_done, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (last) __threadfence();
+    return last;
+}
+
+// f = g + h of every candidate (h as pg_calculate_h: the sum over pairs of the table cell x w); the last block reads the
+// level's f range and starts the select: every candidate is kept when they number at most W, else the bits of f - f_min
+// above the range's highest set bit are decided (all zero) and the W least by (f, key) remain to be found.
+template <int N, int KEYW>
+__global__ void __launch_bounds__(LAY_THREADS) beam_score_kernel(const __grid_constant__ DevProblem p, const __grid_constant__ DevLay d)
+{
+    LayCtrl *c = d.ctrl;
+    if (c->dead || c->error) return;
+    const uint32_t n = c->list_n;
+    const unsigned fmask = (1u << d.kb) - 1u;
+    int lo = INT_MAX, hi = INT_MIN;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const Key<KEYW> k = beam_cand_key<KEYW>(d, i);
+        int pos[N];
+#pragma unroll
+        for (int x = 0; x < N; x++) pos[x] = (int)k.field(x * d.kb, fmask);
+        int h = 0;
+#pragma unroll
+        for (int x = 0; x < N; x++)
+#pragma unroll
+            for (int y = x + 1; y < N; y++) {
+                const int pr = x * N - x * (x + 1) / 2 + (y - x - 1);
+                h += pg_table_cell(p, pr, pos[x], pos[y]) * p.w[pr];
+            }
+        const int f = (int)(d.cand_val[i] >> 32) + h;
+        d.cand_f[i] = f;
+        lo = min(lo, f);
+        hi = max(hi, f);
+    }
+    for (int o = 16; o; o >>= 1) {
+        lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+        hi = max(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+    }
+    if ((threadIdx.x & 31) == 0 && lo != INT_MAX) {
+        atomicMin(&c->lvl_fmin, lo);
+        atomicMax(&c->lvl_fmax, hi);
+    }
+    if (!beam_last_block(c) || threadIdx.x != 0) return;
+    volatile LayCtrl *vc = c;
+    const int f0 = vc->lvl_fmin, f1 = vc->lvl_fmax;
+    const uint32_t k = min(n, d.width);
+    c->lvl_fmin = INT_MAX;
+    c->lvl_fmax = INT_MIN;
+    c->blocks_done = 0;
+    c->cand_n = n;
+    c->max_cand = max(c->max_cand, (unsigned long long)n);
+    c->ret_base = c->ret_n;
+    c->ret_n += k;
+    if (c->ret_n > d.ret_cap) c->error = 1; // the host sized the array for every level: not reached
+    c->dropped += n - k;
+    c->keep_n = 0;
+    c->sel_all = c->sel_done = n <= d.width;
+    c->sel_k = k;
+    c->sel_f0 = f0;
+    const int z = __clz((int)((unsigned)f1 - (unsigned)f0));
+    c->sel_fp = 0;
+    c->sel_fm = z == 0 ? 0u : ~0u << (32 - z);
+    c->sel_kp[0] = c->sel_kp[1] = c->sel_km[0] = c->sel_km[1] = 0;
+}
+
+// The decided bits of the select, in registers: a candidate's (f - f0, key) under the masks against the prefix
+struct BeamSel {
+    unsigned f0, fp, fm;
+    unsigned long long kp[2], km[2];
+    __device__ __forceinline__ explicit BeamSel(const LayCtrl *c)
+        : f0((unsigned)c->sel_f0), fp(c->sel_fp), fm(c->sel_fm), kp{c->sel_kp[0], c->sel_kp[1]}, km{c->sel_km[0], c->sel_km[1]}
+    {
+    }
+    // -1, 0, 1: below, in, above the tie class of the prefix
+    template <int KEYW>
+    __device__ __forceinline__ int cmp(int f, const Key<KEYW> &k) const
+    {
+        const unsigned a = ((unsigned)f - f0) & fm;
+        if (a != fp) return a < fp ? -1 : 1;
+        if constexpr (KEYW == 2) {
+            const unsigned long long h = k.hi & km[1];
+            if (h != kp[1]) return h < kp[1] ? -1 : 1;
+        }
+        const unsigned long long l = k.lo & km[0];
+        return l == kp[0] ? 0 : (l < kp[0] ? -1 : 1);
+    }
+};
+
+// One radix-select pass: digit 0 .. 3 are the bytes of f - f_min from the top, digit 4 + j byte kd - 1 - j of the packed
+// key.  The candidates in the tie class are counted by the digit's value; the last block finds the bin that holds the
+// sel_k-th of them and adds it to the prefix.  When that bin holds exactly the candidates still wanted, the cut is decided.
+template <int KEYW>
+__global__ void __launch_bounds__(LAY_THREADS) beam_select_kernel(const __grid_constant__ DevLay d, int digit)
+{
+    LayCtrl *c = d.ctrl;
+    if (c->dead || c->error || c->sel_done) return;
+    const bool fd = digit < 4;
+    const int sh = fd ? 24 - 8 * digit : 8 * (d.kd - 1 - (digit - 4));
+    if (fd && ((c->sel_fm >> sh) & 0xffu) == 0xffu) return; // decided by the f range
+    __shared__ uint32_t s_h[256];
+    for (int b = threadIdx.x; b < 256; b += blockDim.x) s_h[b] = 0;
+    __syncthreads();
+    const uint32_t n = c->cand_n;
+    const BeamSel sel(c);
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const int f = d.cand_f[i];
+        const Key<KEYW> k = beam_cand_key<KEYW>(d, i);
+        if (sel.cmp<KEYW>(f, k) != 0) continue;
+        unsigned long long word = (unsigned)f - sel.f0;
+        if (!fd) {
+            word = k.lo;
+            if constexpr (KEYW == 2)
+                if (sh >= 64) word = k.hi;
+        }
+        const uint32_t v = (uint32_t)(word >> (sh & 63)) & 0xffu;
+        atomicAdd(s_h + v, 1u);
+    }
+    __syncthreads();
+    for (int b = threadIdx.x; b < 256; b += blockDim.x)
+        if (s_h[b]) atomicAdd(d.sel_hist + b, s_h[b]);
+    if (!beam_last_block(c) || threadIdx.x != 0) return;
+    volatile uint32_t *h = d.sel_hist;
+    const uint32_t want = c->sel_k;
+    uint32_t below = 0, b = 0;
+    for (; b < 255 && below + h[b] < want; b++) below += h[b];
+    const uint32_t rest = want - below;
+    if (fd) {
+        c->sel_fp |= b << sh;
+        c->sel_fm |= 0xffu << sh;
+    } else {
+        c->sel_kp[sh >> 6] |= (unsigned long long)b << (sh & 63);
+        c->sel_km[sh >> 6] |= 0xffull << (sh & 63);
+    }
+    c->sel_k = rest;
+    if (h[b] == rest) c->sel_done = 1;
+    for (int i = 0; i < 256; i++) h[i] = 0;
+    c->blocks_done = 0;
+}
+
+// The kept candidates (all, or those whose decided bits are at most the prefix) to the expand list and the retained
+// array; the least f of the dropped ones to drop_fmin.
+template <int KEYW>
+__global__ void __launch_bounds__(LAY_THREADS) beam_keep_kernel(const __grid_constant__ DevLay d)
+{
+    LayCtrl *c = d.ctrl;
+    if (c->dead || c->error) return;
+    const uint32_t n = c->cand_n;
+    const bool all = c->sel_all;
+    const BeamSel sel(c);
+    const unsigned long long base = c->ret_base;
+    const int lane = threadIdx.x & 31;
+    int dmin = INT_MAX;
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t i0 = blockIdx.x * blockDim.x; i0 < n; i0 += stride) { // warp-uniform trip count
+        const uint32_t i = i0 + threadIdx.x;
+        bool keep = false;
+        Key<KEYW> k = Key<KEYW>::zero();
+        unsigned long long v = 0;
+        if (i < n) {
+            const int f = d.cand_f[i];
+            k = beam_cand_key<KEYW>(d, i);
+            v = d.cand_val[i];
+            keep = all || sel.cmp<KEYW>(f, k) <= 0;
+            if (!keep) dmin = min(dmin, f);
+        }
+        const unsigned ball = __ballot_sync(0xffffffffu, keep);
+        uint32_t at = 0;
+        if (lane == 0 && ball) at = atomicAdd(&c->keep_n, (uint32_t)__popc(ball));
+        at = __shfl_sync(0xffffffffu, at, 0) + __popc(ball & ((1u << lane) - 1u));
+        if (keep) {
+            const unsigned long long r = base + at;
+            d.list_key[at] = k.lo;
+            d.ret_key[r] = k.lo;
+            if constexpr (KEYW == 2) {
+                d.list_key[d.L + at] = k.hi;
+                d.ret_key[d.ret_cap + r] = k.hi;
+            }
+            d.list_val[at] = (v & 0xffffffff00000000ull) | (uint32_t)r;
+            d.ret_val[r] = v;
+        }
+    }
+    for (int o = 16; o; o >>= 1) dmin = min(dmin, __shfl_xor_sync(0xffffffffu, dmin, o));
+    if (lane == 0 && dmin != INT_MAX) atomicMin(&c->drop_fmin, dmin);
+    if (blockIdx.x == 0 && threadIdx.x == 0) c->list_n = min(n, d.width); // the expand kernel's count; n stays in cand_n
+}
+
+// The moves from the origin to t: from the retained entry `at` (t's parent) along the parent indices.  out[0] = moves
+// (~0 when the chain breaks), out[1] unused, out[2 ..] = the masks, t first.
+template <int KEYW>
+__global__ void beam_trace_kernel(const __grid_constant__ DevLay d, uint32_t at, uint32_t *out, int max_moves)
+{
+    int cur[PG_MAX_SEQ];
+    for (int i = 0; i < d.n; i++) cur[i] = d.t[i];
+    const unsigned fmask = (1u << d.kb) - 1u;
+    int k = 0;
+    out[0] = ~0u;
+    for (; at != ~0u; k++) {
+        if (k >= max_moves || at >= d.ret_cap) return;
+        Key<KEYW> key;
+        key.lo = d.ret_key[at];
+        if constexpr (KEYW == 2) key.hi = d.ret_key[d.ret_cap + at];
+        uint32_t m = 0;
+        for (int i = 0; i < d.n; i++) {
+            const int q = (int)key.field(i * d.kb, fmask), step = cur[i] - q;
+            if (step != 0 && step != 1) return;
+            m |= (uint32_t)step << i;
+            cur[i] = q;
+        }
+        if (m == 0) return;
+        out[2 + k] = m;
+        at = (uint32_t)d.ret_val[at];
+    }
+    for (int i = 0; i < d.n; i++)
+        if (cur[i] != d.s[i]) return;
+    out[0] = (uint32_t)k;
+}
+
 template <int N, int KEYW>
 size_t expand_smem()
 {
@@ -386,6 +654,14 @@ template <int N, int KEYW>
 int launch_level_expand(pg_ctx *ctx, const DevLay &d, int grid)
 {
     layered_expand_kernel<N, KEYW><<<grid, LAY_THREADS, expand_smem<N, KEYW>(), ctx->stream>>>(ctx->dp, d);
+    PG_CUDA(ctx, cudaGetLastError());
+    return PG_OK;
+}
+
+template <int N, int KEYW>
+int launch_beam_score(pg_ctx *ctx, const DevLay &d, int grid)
+{
+    beam_score_kernel<N, KEYW><<<grid, LAY_THREADS, 0, ctx->stream>>>(ctx->dp, d);
     PG_CUDA(ctx, cudaGetLastError());
     return PG_OK;
 }
@@ -411,6 +687,11 @@ struct LayeredState {
     unsigned long long *keys = nullptr, *vals = nullptr, *list_key = nullptr, *list_val = nullptr, *relay_key = nullptr,
                        *relay_val = nullptr, *hist = nullptr;
     uint32_t *claims = nullptr, *counts = nullptr, *trace = nullptr;
+    // beam mode: the candidates before the cut, the select's bins, the retained array and the trace's output
+    unsigned long long *cand_key = nullptr, *cand_val = nullptr, *ret_key = nullptr, *ret_val = nullptr;
+    int32_t *cand_f = nullptr;
+    uint32_t *sel_hist = nullptr, *beam_trace = nullptr;
+    int64_t ret_cap = 0;
     LayCtrl *d_ctrl = nullptr, *h_ctrl = nullptr;
     int64_t bytes = 0;
     int expand_grid = 0, compact_grid = 0;
@@ -424,6 +705,22 @@ int lay_alloc(pg_ctx *ctx, LayeredState *L, void **p, size_t bytes)
     PG_CUDA(ctx, cudaMalloc(p, bytes));
     L->bytes += (int64_t)bytes;
     return PG_OK;
+}
+
+int beam_score(pg_ctx *ctx, const DevLay &d, int grid)
+{
+    const int kw = ctx->n * ctx->dp.key_bits <= 63 ? 1 : 2;
+    switch (ctx->n * 2 + kw - 1) {
+#define CASE(X)                                                                                                   \
+    case 2 * X:                                                                                                   \
+        return launch_beam_score<X, 1>(ctx, d, grid);                                                             \
+    case 2 * X + 1:                                                                                               \
+        return launch_beam_score<X, 2>(ctx, d, grid);
+        CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8) CASE(9) CASE(10) CASE(11) CASE(12) CASE(13) CASE(14) CASE(15) CASE(16)
+#undef CASE
+    default:
+        return pg_fail(ctx, PG_ERR_ARG, "pg_search_beam: unsupported number of sequences");
+    }
 }
 
 int lay_expand(pg_ctx *ctx, const DevLay &d, int grid, bool attr_only, int *grid_out)
@@ -475,17 +772,65 @@ DevLay make_dev(const pg_ctx *ctx, const LayeredState *L, const LayPassIn &in)
     d.hist_w = std::max(1, in.hist_w);
     d.hist = L->hist;
     d.ctrl = L->d_ctrl;
+    d.width = (uint32_t)std::min<int64_t>(in.width, UINT32_MAX);
+    d.kd = (ctx->n * ctx->dp.key_bits + 7) / 8;
+    d.cand_key = L->cand_key;
+    d.cand_val = L->cand_val;
+    d.cand_f = L->cand_f;
+    d.sel_hist = L->sel_hist;
+    d.ret_key = L->ret_key;
+    d.ret_val = L->ret_val;
+    d.ret_cap = (unsigned long long)L->ret_cap;
     return d;
+}
+
+// the view the compact kernel writes through: in beam mode the level goes to the candidate list, not the expand list
+DevLay compact_view(const DevLay &d)
+{
+    DevLay c = d;
+    if (d.width) {
+        c.list_key = d.cand_key;
+        c.list_val = d.cand_val;
+    }
+    return c;
+}
+
+int launch_compact(pg_ctx *ctx, const LayeredState *L, const DevLay &d, int grid)
+{
+    const DevLay c = compact_view(d);
+    if (L->keyw == 1)
+        layered_compact_kernel<1><<<grid, LAY_THREADS, 0, ctx->stream>>>(c);
+    else
+        layered_compact_kernel<2><<<grid, LAY_THREADS, 0, ctx->stream>>>(c);
+    PG_CUDA(ctx, cudaGetLastError());
+    return PG_OK;
+}
+
+// the cut of the compacted level: score, one select pass per digit (4 of f, kd of the key), keep
+int launch_cut(pg_ctx *ctx, const LayeredState *L, const DevLay &d)
+{
+    int rc = beam_score(ctx, d, L->compact_grid);
+    if (rc != PG_OK) return rc;
+    for (int digit = 0; digit < 4 + d.kd; digit++) {
+        if (L->keyw == 1)
+            beam_select_kernel<1><<<L->compact_grid, LAY_THREADS, 0, ctx->stream>>>(d, digit);
+        else
+            beam_select_kernel<2><<<L->compact_grid, LAY_THREADS, 0, ctx->stream>>>(d, digit);
+    }
+    if (L->keyw == 1)
+        beam_keep_kernel<1><<<L->compact_grid, LAY_THREADS, 0, ctx->stream>>>(d);
+    else
+        beam_keep_kernel<2><<<L->compact_grid, LAY_THREADS, 0, ctx->stream>>>(d);
+    PG_CUDA(ctx, cudaGetLastError());
+    return PG_OK;
 }
 
 int launch_level(pg_ctx *ctx, const LayeredState *L, const DevLay &d)
 {
-    if (L->keyw == 1)
-        layered_compact_kernel<1><<<L->compact_grid, LAY_THREADS, 0, ctx->stream>>>(d);
-    else
-        layered_compact_kernel<2><<<L->compact_grid, LAY_THREADS, 0, ctx->stream>>>(d);
-    PG_CUDA(ctx, cudaGetLastError());
-    int rc = lay_expand(ctx, d, L->expand_grid, false, nullptr);
+    int rc = launch_compact(ctx, L, d, L->compact_grid);
+    if (rc == PG_OK && d.width) rc = launch_cut(ctx, L, d);
+    if (rc != PG_OK) return rc;
+    rc = lay_expand(ctx, d, L->expand_grid, false, nullptr);
     if (rc != PG_OK) return rc;
     layered_advance_kernel<<<1, 1, 0, ctx->stream>>>(d);
     PG_CUDA(ctx, cudaGetLastError());
@@ -501,7 +846,7 @@ int read_ctrl(pg_ctx *ctx, LayeredState *L)
 
 } // namespace
 
-int pg_layered_open(pg_ctx *ctx, int64_t level_cap, int retain_levels, LayeredState **out)
+int pg_layered_open(pg_ctx *ctx, int64_t level_cap, int retain_levels, int64_t beam_retained, LayeredState **out)
 {
     *out = nullptr;
     LayeredState *L = new LayeredState();
@@ -512,17 +857,40 @@ int pg_layered_open(pg_ctx *ctx, int64_t level_cap, int retain_levels, LayeredSt
     while ((1LL << L->lg_s) < 2 * L->L) L->lg_s++; // load factor at most one half
     L->n_tables = std::max(ctx->n + 1, retain_levels);
     L->no_graph = getenv("PG_NO_GRAPH") != nullptr;
+    L->ret_cap = beam_retained;
     *out = L;
     const size_t S = (size_t)1 << L->lg_s, T = (size_t)L->n_tables;
     int rc;
+    if (beam_retained > 0) {
+        int D = 0;
+        for (int i = 0; i < ctx->n; i++) D += ctx->len[i];
+        const size_t kw = (size_t)L->keyw, Lc = (size_t)L->L, R = (size_t)beam_retained;
+        const size_t need = T * S * kw * 8 + T * S * 8 + T * Lc * 4 + T * 4 + 2 * (Lc * kw * 8 + Lc * 8) + Lc * 4 + 256 * 4 +
+                            R * (kw * 8 + 8) + ((size_t)D + 2) * 4 + LAY_NB * 8 + ((size_t)T + 2) * 4 + sizeof(LayCtrl);
+        size_t free_b = 0, total_b = 0;
+        PG_CUDA(ctx, cudaMemGetInfo(&free_b, &total_b));
+        if (need > free_b)
+            return pg_fail(ctx, PG_ERR_CAPACITY, "pg_search_beam: " + std::to_string(need) + " bytes of level tables and retained array, " +
+                                                     std::to_string(free_b) + " free on the device");
+        if ((rc = lay_alloc(ctx, L, (void **)&L->cand_key, Lc * kw * 8)) != PG_OK) return rc;
+        if ((rc = lay_alloc(ctx, L, (void **)&L->cand_val, Lc * 8)) != PG_OK) return rc;
+        if ((rc = lay_alloc(ctx, L, (void **)&L->cand_f, Lc * 4)) != PG_OK) return rc;
+        if ((rc = lay_alloc(ctx, L, (void **)&L->sel_hist, 256 * 4)) != PG_OK) return rc;
+        if ((rc = lay_alloc(ctx, L, (void **)&L->ret_key, R * kw * 8)) != PG_OK) return rc;
+        if ((rc = lay_alloc(ctx, L, (void **)&L->ret_val, R * 8)) != PG_OK) return rc;
+        if ((rc = lay_alloc(ctx, L, (void **)&L->beam_trace, ((size_t)D + 2) * 4)) != PG_OK) return rc;
+        PG_CUDA(ctx, cudaMemsetAsync(L->sel_hist, 0, 256 * 4, ctx->stream));
+    }
     if ((rc = lay_alloc(ctx, L, (void **)&L->keys, T * S * L->keyw * 8)) != PG_OK) return rc;
     if ((rc = lay_alloc(ctx, L, (void **)&L->vals, T * S * 8)) != PG_OK) return rc;
     if ((rc = lay_alloc(ctx, L, (void **)&L->claims, T * L->L * 4)) != PG_OK) return rc;
     if ((rc = lay_alloc(ctx, L, (void **)&L->counts, T * 4)) != PG_OK) return rc;
     if ((rc = lay_alloc(ctx, L, (void **)&L->list_key, (size_t)L->L * L->keyw * 8)) != PG_OK) return rc;
     if ((rc = lay_alloc(ctx, L, (void **)&L->list_val, (size_t)L->L * 8)) != PG_OK) return rc;
-    if ((rc = lay_alloc(ctx, L, (void **)&L->relay_key, (size_t)L->L * ctx->n * L->keyw * 8)) != PG_OK) return rc;
-    if ((rc = lay_alloc(ctx, L, (void **)&L->relay_val, (size_t)L->L * ctx->n * 8)) != PG_OK) return rc;
+    if (beam_retained == 0) { // beam passes have no relays
+        if ((rc = lay_alloc(ctx, L, (void **)&L->relay_key, (size_t)L->L * ctx->n * L->keyw * 8)) != PG_OK) return rc;
+        if ((rc = lay_alloc(ctx, L, (void **)&L->relay_val, (size_t)L->L * ctx->n * 8)) != PG_OK) return rc;
+    }
     if ((rc = lay_alloc(ctx, L, (void **)&L->hist, LAY_NB * 8)) != PG_OK) return rc;
     if ((rc = lay_alloc(ctx, L, (void **)&L->trace, ((size_t)T + 2) * 4)) != PG_OK) return rc;
     if ((rc = lay_alloc(ctx, L, (void **)&L->d_ctrl, sizeof(LayCtrl))) != PG_OK) return rc;
@@ -542,7 +910,9 @@ void pg_layered_close(pg_ctx *ctx, LayeredState *L)
     if (!L) return;
     cudaStreamSynchronize(ctx->stream);
     for (void *p : {(void *)L->keys, (void *)L->vals, (void *)L->claims, (void *)L->counts, (void *)L->list_key, (void *)L->list_val,
-                    (void *)L->relay_key, (void *)L->relay_val, (void *)L->hist, (void *)L->trace, (void *)L->d_ctrl})
+                    (void *)L->relay_key, (void *)L->relay_val, (void *)L->hist, (void *)L->trace, (void *)L->d_ctrl,
+                    (void *)L->cand_key, (void *)L->cand_val, (void *)L->cand_f, (void *)L->sel_hist, (void *)L->ret_key,
+                    (void *)L->ret_val, (void *)L->beam_trace})
         cudaFree(p);
     if (L->h_ctrl) cudaFreeHost(L->h_ctrl);
     delete L;
@@ -557,10 +927,14 @@ int pg_layered_pass(pg_ctx *ctx, LayeredState *L, const LayPassIn &in, int64_t b
     if (d.nt > L->n_tables) return pg_fail(ctx, PG_ERR_STATE, "pg_search_layered: a retain pass wider than its tables");
     PG_CUDA(ctx, cudaMemsetAsync(L->d_ctrl, 0, sizeof(LayCtrl), ctx->stream));
     PG_CUDA(ctx, cudaMemsetAsync(L->hist, 0, LAY_NB * 8, ctx->stream));
+    if (d.width && L->ret_cap <= 0)
+        return pg_fail(ctx, PG_ERR_STATE, "pg_search_beam: the level tables were opened without a retained array");
+    // the origin's low: its parent in beam mode (none), the all-ones move in retain mode, no relay yet in relay mode
+    const uint32_t low0 = d.width ? ~0u : (d.retain ? (1u << d.n) - 1u : RELAY_BASE);
     if (L->keyw == 1)
-        layered_seed_kernel<1><<<1, 1, 0, ctx->stream>>>(d, in.g0);
+        layered_seed_kernel<1><<<1, 1, 0, ctx->stream>>>(d, in.g0, low0);
     else
-        layered_seed_kernel<2><<<1, 1, 0, ctx->stream>>>(d, in.g0);
+        layered_seed_kernel<2><<<1, 1, 0, ctx->stream>>>(d, in.g0, low0);
     PG_CUDA(ctx, cudaGetLastError());
 
     // levels ls .. lt - 1, checked every LAY_SYNC levels; groups of LAY_GROUP levels replay one captured graph
@@ -600,17 +974,12 @@ int pg_layered_pass(pg_ctx *ctx, LayeredState *L, const LayPassIn &in, int64_t b
         }
     }
     // level lt: t alone (the box's last corner)
-    if (!out.aborted) {
-        if (L->keyw == 1)
-            layered_compact_kernel<1><<<1, LAY_THREADS, 0, ctx->stream>>>(d);
-        else
-            layered_compact_kernel<2><<<1, LAY_THREADS, 0, ctx->stream>>>(d);
-        PG_CUDA(ctx, cudaGetLastError());
-    }
+    if (!out.aborted && (rc = launch_compact(ctx, L, d, 1)) != PG_OK) return rc;
     if ((rc = read_ctrl(ctx, L)) != PG_OK) return rc;
     const LayCtrl c = *L->h_ctrl;
-    if (c.error) return pg_fail(ctx, PG_ERR_CAPACITY, "pg_search_layered: a level holds more than " + std::to_string(L->L) +
-                                                          " coordinates (raise table_capacity)");
+    if (c.error)
+        return pg_fail(ctx, PG_ERR_CAPACITY, std::string(d.width ? "pg_search_beam" : "pg_search_layered") + ": a level holds more than " +
+                                                 std::to_string(L->L) + " coordinates (raise table_capacity)");
     out.fmin = c.fmin;
     out.fmax = c.fmax;
     out.expansions = (int64_t)c.expansions;
@@ -619,15 +988,20 @@ int pg_layered_pass(pg_ctx *ctx, LayeredState *L, const LayPassIn &in, int64_t b
     out.levels = (int64_t)c.levels;
     out.max_level_nodes = (int64_t)c.max_level;
     out.max_held = (int64_t)c.max_held;
+    out.kept = (int64_t)c.ret_n;
+    out.dropped = (int64_t)c.dropped;
+    out.max_cand = (int64_t)c.max_cand;
+    out.drop_fmin = c.drop_fmin;
     out.hist.assign(LAY_NB, 0);
     PG_CUDA(ctx, cudaMemcpyAsync(out.hist.data(), L->hist, LAY_NB * 8, cudaMemcpyDeviceToHost, ctx->stream));
     if (!out.aborted && !c.dead && c.d == d.lt && c.list_n == 1) {
         unsigned long long v = 0;
-        PG_CUDA(ctx, cudaMemcpyAsync(&v, L->list_val, 8, cudaMemcpyDeviceToHost, ctx->stream));
+        PG_CUDA(ctx, cudaMemcpyAsync(&v, d.width ? L->cand_val : L->list_val, 8, cudaMemcpyDeviceToHost, ctx->stream));
         PG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         out.reached = true;
         out.goal_g = (int)(v >> 32);
-        if (!in.retain) {
+        out.goal_parent = (uint32_t)v;
+        if (!in.retain && !d.width) {
             const uint32_t low = (uint32_t)v;
             if (low < RELAY_BASE) return pg_fail(ctx, PG_ERR_STATE, "pg_search_layered: t has no relay");
             const size_t id = low - RELAY_BASE, cap = (size_t)L->L * ctx->n;
@@ -676,6 +1050,24 @@ int pg_layered_trace(pg_ctx *ctx, LayeredState *L, const LayPassIn &in, std::vec
     PG_CUDA(ctx, cudaGetLastError());
     PG_CUDA(ctx, cudaMemsetAsync(L->counts, 0, (size_t)d.nt * 4, ctx->stream));
     if (tr[0] == ~0u) return pg_fail(ctx, PG_ERR_STATE, "pg_search_layered: the retained levels lost the parent chain");
+    masks.resize(tr[0]);
+    for (uint32_t k = 0; k < tr[0]; k++) masks[k] = tr[2 + (tr[0] - 1 - k)]; // stored t first
+    return PG_OK;
+}
+
+int pg_beam_trace(pg_ctx *ctx, LayeredState *L, const LayPassIn &in, uint32_t goal_parent, std::vector<uint32_t> &masks)
+{
+    const DevLay d = make_dev(ctx, L, in);
+    const int max_moves = d.lt - d.ls;
+    if (L->keyw == 1)
+        beam_trace_kernel<1><<<1, 1, 0, ctx->stream>>>(d, goal_parent, L->beam_trace, max_moves);
+    else
+        beam_trace_kernel<2><<<1, 1, 0, ctx->stream>>>(d, goal_parent, L->beam_trace, max_moves);
+    PG_CUDA(ctx, cudaGetLastError());
+    std::vector<uint32_t> tr((size_t)max_moves + 2);
+    PG_CUDA(ctx, cudaMemcpyAsync(tr.data(), L->beam_trace, tr.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (tr[0] == ~0u) return pg_fail(ctx, PG_ERR_STATE, "pg_search_beam: the retained parents do not lead back to the origin");
     masks.resize(tr[0]);
     for (uint32_t k = 0; k < tr[0]; k++) masks[k] = tr[2 + (tr[0] - 1 - k)]; // stored t first
     return PG_OK;
